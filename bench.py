@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl clipk|reference]
                     [--config c2|c3|c4] [--mode local|global] [--gwg 0|1] [--logit-scale S] [--skip-extras]
+                    [--dump-outputs DIR]
 
 One process per GPU (under torchrun for N > 1; RANK / LOCAL_RANK / WORLD_SIZE from the environment).  The global batch
 is fixed, so the N-GPU runs are a strong-scaling series: each rank owns global_batch / N rows.
@@ -17,7 +18,9 @@ What one run does, in order (rank 0 prints ONE JSON line at the end):
      benchmark's own shapes through the very ClipLoss call that is timed, against a chunked fp32 torch evaluation of the
      reference formula on the same GPU(s).  A failure is reported in the line and the process exits non-zero.
   2. `value`: K steps with the inputs resident in HBM, every step inside its own CUDA event pair, a 256 MiB L2 flush
-     between steps (outside the pairs), max over ranks.
+     between steps (outside the pairs), max over ranks.  With --dump-outputs DIR, rank 0 then writes what the last of
+     these steps returned as float32 DIR/<name>.npy: loss, d_logit_scale, and d_image / d_text, each cut to a seeded
+     sample of 16 MB of rows when larger.  The inputs are seeded, so two builds can be compared file by file.
   3. `e2e`: the same call fed from pinned host buffers (H2D of both feature matrices and D2H of the loss inside the timed
      region); `serial_*` is the conservative single-stream figure, the headline prefetches the next step's inputs.
   4. per-kernel times of one rank's step from the library's own event profile -> roofline of the dominant kernel.
@@ -51,6 +54,7 @@ METRIC = "ClipLoss fwd+bwd samples/s @ global batch 32K, d=512"
 CPU_SAMPLE_BATCH = 8192           # calibration size of the CPU arms (cost grows with batch^2)
 CPU_ARM_BUDGET_S = 240.0          # whole `--impl reference` run
 REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+DUMP_MATRIX_BYTES = 16 << 20      # per gradient matrix written by --dump-outputs (as float32)
 
 
 def peaks():
@@ -348,6 +352,21 @@ def parse_profile(text):
     return out
 
 
+def dump_outputs(out_dir, tensors):
+    """--dump-outputs: each tensor as float32 <out_dir>/<name>.npy.  A matrix larger than DUMP_MATRIX_BYTES is cut to
+    a seeded sample of its rows (sorted; the same rows for the same shape), which keeps the dump under 64 MB."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in tensors.items():
+        t = t.detach()
+        if t.dim() == 2 and t.numel() * 4 > DUMP_MATRIX_BYTES:
+            rows = DUMP_MATRIX_BYTES // (4 * t.shape[1])
+            idx = np.sort(np.random.default_rng(0).choice(t.shape[0], rows, replace=False))
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_clipk(args):
     import torch
     import torch.distributed as dist
@@ -487,6 +506,8 @@ def run_clipk(args):
         loss_host.copy_(loss.detach(), non_blocking=True)
         return loss
 
+    last_out = {}       # what the last timed step returned (--dump-outputs)
+
     def timed(fn, steps, warmup):
         for _ in range(warmup):
             fn()
@@ -501,7 +522,7 @@ def run_clipk(args):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             la = ops.gpu_launches()
             e0.record()
-            fn()
+            last_out["loss"] = fn()
             e1.record()
             launches += ops.gpu_launches() - la
             pairs.append((e0, e1))
@@ -565,6 +586,9 @@ def run_clipk(args):
     if sampler:
         sampler.start()
     ms, launches, host_ms = timed(step_resident, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": last_out["loss"].detach(), "d_image": I.grad, "d_text": T.grad,
+                                         "d_logit_scale": S.grad})
     loss_resident = float(step_resident().detach())
     single_sweep = ops.last_forward_was_single_sweep()
     e2e_steps = max(3, args.steps // 2)
@@ -837,7 +861,13 @@ def main():
     ap.add_argument("--gwg", type=int, default=None, choices=[0, 1])
     ap.add_argument("--logit-scale", type=float, default=INIT_SCALE)
     ap.add_argument("--skip-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and gradients of the last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "clipk":
+        ap.error("--dump-outputs applies to --impl clipk")
     args.warmup = max(args.warmup, 3) if args.impl == "clipk" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -185,17 +185,17 @@ class TorchPort:
     def __init__(self):
         self._labels = None
 
-    def labels(self, n: int):
+    def labels(self, n: int, device=None):
         import torch
-        if self._labels is None or self._labels.numel() != n:
-            self._labels = torch.arange(n, dtype=torch.long)
+        if self._labels is None or self._labels.numel() != n or self._labels.device != torch.device(device or "cpu"):
+            self._labels = torch.arange(n, dtype=torch.long, device=device)
         return self._labels
 
     def __call__(self, image_features, text_features, logit_scale):
         import torch.nn.functional as F
         a = logit_scale * image_features @ text_features.T
         b = logit_scale * text_features @ image_features.T
-        y = self.labels(a.shape[0])
+        y = self.labels(a.shape[0], a.device)
         return (F.cross_entropy(a, y) + F.cross_entropy(b, y)) / 2
 
     def fwd_bwd(self, image_features, text_features, logit_scale):

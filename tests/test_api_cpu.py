@@ -309,6 +309,27 @@ def test_bench_reference_arm_prints_one_json_line():
     assert j["e2e"]["h2d_bytes_per_step"] == 0 and j["e2e"]["d2h_bytes_per_step"] == 0 and j["value"] > 0
 
 
+def test_bench_dump_outputs_writes_float32_with_a_seeded_row_sample(tmp_path):
+    """`bench.py --dump-outputs`: float32 .npy per output; a matrix above the budget becomes the same sorted row sample
+    on every call, so that dumps of two builds line up row for row."""
+    import bench
+    g = torch.Generator().manual_seed(0)
+    rows = bench.DUMP_MATRIX_BYTES // (4 * 64)
+    big = torch.randn(3 * rows, 64, generator=g).bfloat16()
+    small = torch.randn(rows, 64, generator=g).bfloat16()
+    for out in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / out), {"loss": torch.tensor(1.5), "big": big, "small": small})
+    a = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("loss", "big", "small")}
+    assert all(v.dtype == np.float32 for v in a.values())
+    assert a["loss"].shape == () and float(a["loss"]) == 1.5
+    assert np.array_equal(a["small"], small.float().numpy())
+    assert a["big"].shape == (rows, 64) and a["big"].nbytes <= bench.DUMP_MATRIX_BYTES
+    assert np.array_equal(a["big"], np.load(tmp_path / "b" / "big.npy"))
+    full = big.float().numpy()
+    idx = [int(np.flatnonzero((full == r).all(axis=1))[0]) for r in a["big"][:50]]
+    assert idx == sorted(set(idx))                  # distinct rows of the input, in order
+
+
 @pytest.mark.parametrize("n,d,s", [(96, 48, 1 / 0.07), (130, 32, 100.0)])
 def test_bench_parity_checker_matches_the_oracle(n, d, s):
     """bench.py's parity phase checks the benchmark's own shapes against `torch_fp32_reference` (chunked fp32 torch, no

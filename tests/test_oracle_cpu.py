@@ -59,6 +59,20 @@ def test_torch_port_matches_oracle():
     assert abs(float(ds) - ref.d_scale) < 1e-4 * abs(ref.d_scale)
 
 
+@pytest.mark.gpu
+def test_torch_port_on_cuda_tensors():
+    """bench.py times the port on the GPU as the eager baseline: its labels must follow the logits to the device."""
+    import torch
+    x, t = O.synthetic_features(64, 48, seed=3)
+    port = O.TorchPort()
+    port.fwd_bwd(torch.from_numpy(x), torch.from_numpy(t), torch.tensor(1 / 0.07))      # a CPU call first: labels cached there
+    loss, dI, dT, ds = port.fwd_bwd(torch.from_numpy(x).cuda(), torch.from_numpy(t).cuda(), torch.tensor(1 / 0.07).cuda())
+    ref = O.clip_loss_single(x, t, 1 / 0.07)
+    assert loss.is_cuda and abs(float(loss) - ref.loss) < 1e-4 * abs(ref.loss)
+    assert np.linalg.norm(dI.cpu().numpy() - ref.d_image) < 1e-4 * np.linalg.norm(ref.d_image)
+    assert np.linalg.norm(dT.cpu().numpy() - ref.d_text) < 1e-4 * np.linalg.norm(ref.d_text)
+
+
 def test_bf16_rounding_helper():
     import torch
     x = np.random.default_rng(0).standard_normal(1000).astype(np.float32)
