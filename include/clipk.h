@@ -275,8 +275,8 @@ int clipk_rank_count(const float* S, int rows, int cols, long long ld, const lon
  *                                               + exp(S - s_lse_col[j]) - exp(T - t_lse_col[j]) ) ),  G is [rows, ldg]:
  *                        the derivative of both directions' terms with respect to the student's logits times 2 n,
  *                        in the operand format of the gradient GEMMs (clipk_gemm16 with f16 = 1).
- * rows <= 65535 per call.  STATUS: built and covered on the CPU emulation; GPU validation pending (opt-in,
- * CLIPK_FUSED_DISTILL=1). */
+ * rows <= 65535 per call.  STATUS: validated on a B200 (tests/test_distill_gpu.py) and on the CPU emulation; the
+ * default path of clipk/distill.py for the shapes it accepts (CLIPK_FUSED_DISTILL=0 switches it off). */
 int clipk_distill_cross(const float* S, const float* T, int rows, int cols, long long ld, const float* s_mul,
                         const float* t_mul, const float* t_lse_row, const float* t_lse_col, long long row0,
                         float* row_cross, float* col_part, void* stream);
