@@ -31,12 +31,6 @@ def _panel_rows(rows, cols4, panel_bytes):
     return min(per, rows, 65535 // 256 * 256)
 
 
-def _pad_width(x):
-    """Zero columns up to whole 64-element K blocks (they change no logit; their gradient columns are dropped)."""
-    k = ops._round_up(x.shape[1], ops._K_BLOCK)
-    return x.contiguous() if k == x.shape[1] else torch.nn.functional.pad(x, (0, k - x.shape[1]))
-
-
 class _Model:
     """One model's side of the term: operands, log-sum-exps and the scalar that turns raw panel products into logits."""
 
@@ -44,7 +38,7 @@ class _Model:
         dev = image.device
         n = image.shape[0]
         self.scale = scale.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
-        self.image, self.text = _pad_width(image), _pad_width(text)
+        self.image, self.text = ops._kernel_features(image), ops._kernel_features(text)
         X, Y = be.prepare(self.image), be.prepare(self.text)
         parts = torch.empty(1, 3, n, dtype=torch.float32, device=dev)
         row_stats, pos, _ = be.fwd_both(X, Y, self.scale, 0, col_out=parts[0])
@@ -131,9 +125,7 @@ def applicable(image_features, text_features, dist_image_features, dist_text_fea
         return False
     if image_features.shape != text_features.shape or dist_image_features.shape != dist_text_features.shape:
         return False
-    dev = image_features.device
-    autocast_bf16 = dev.type == "cuda" and torch.is_autocast_enabled("cuda") and \
-        torch.get_autocast_dtype("cuda") == torch.bfloat16
+    autocast_bf16 = ops._autocast_bf16(image_features.device)
     return all(f.dtype == torch.bfloat16 or (autocast_bf16 and f.dtype == torch.float32) for f in feats)
 
 

@@ -36,13 +36,7 @@ class _IctLoss(torch.autograd.Function):
         N = world * b
         dev = query.device
         in_dtype = query.dtype
-        q, c = query.detach(), context.detach()
-        if in_dtype == torch.float16:
-            q, c = q.float(), c.float()
-        d = ops._round_up(d_in, ops._K_BLOCK)
-        if d != d_in:
-            q = torch.nn.functional.pad(q, (0, d - d_in))
-            c = torch.nn.functional.pad(c, (0, d - d_in))
+        q, c = ops._kernel_features(query.detach()), ops._kernel_features(context.detach())
         scale = torch.tensor([float(score_scale)], dtype=torch.float32, device=dev)
         q_all = _all_gather_rows(q, world, group) if world > 1 else q
         c_all = _all_gather_rows(c, world, group) if world > 1 else c
@@ -59,7 +53,7 @@ class _IctLoss(torch.autograd.Function):
         loss = part[0] / N * world
         ctx.save_for_backward(query, context, scale, lse, lse_all)
         ctx.operands = (Xq, Xc, Yq, Yc)
-        ctx.cfg = (b, d, d_in, N, off, world, in_dtype)
+        ctx.cfg = (b, d_in, off, world, in_dtype)
         ctx.pos = pos
         return loss
 
@@ -69,8 +63,7 @@ class _IctLoss(torch.autograd.Function):
         be = ops._backend()
         _, _, scale, lse, lse_all = ctx.saved_tensors
         Xq, Xc, Yq, Yc = ctx.operands
-        b, d, d_in, N, off, world, in_dtype = ctx.cfg
-        k_dtype = torch.bfloat16 if in_dtype == torch.bfloat16 else torch.float32
+        b, d_in, off, world, in_dtype = ctx.cfg
         # d loss / d S_ij = W / N * (P - Id)_ij = (P - Id)_ij / b
         gscale = (grad_out.detach().to(torch.float32).reshape(1) / b).contiguous()
         Gq, Gc = be.prepare_grad(Xq), be.prepare_grad(Xc)
@@ -83,16 +76,8 @@ class _IctLoss(torch.autograd.Function):
             # block [b contexts x N queries] = the transposed column block: the softmax runs over ITS columns' index, so
             # the log-sum-exps of all N queries take the column slot: alpha = 0, beta = 1
             dc, _ = be.bwd(Xc, Yq, Gc, GYq, scale, off, lse, lse_all, 0.0, 1.0, gscale, True, False)
-        outs = []
-        for g in (dq, dc):
-            if g is None:
-                outs.append(None)
-                continue
-            if d != d_in:
-                g = g[:, :d_in].contiguous()
-            g = be.cast(g, k_dtype)
-            outs.append(g if k_dtype == in_dtype else g.to(in_dtype))
-        return outs[0], outs[1], None, None, None, None
+        dq, dc = (None if g is None else ops._caller_grad(be, g, d_in, in_dtype) for g in (dq, dc))
+        return dq, dc, None, None, None, None
 
 
 def ict_retrieval_loss(query_logits, context_logits, retriever_score_scaling=False, hidden_size=None, group=None,

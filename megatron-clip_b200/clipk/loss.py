@@ -10,8 +10,8 @@ Same names, constructor arguments, method signatures and return conventions as t
     CoCaLoss, DistillClipLoss                            reference loss.py:143-221
     create_loss(args)                                    reference factory.py:250-278
 
-`ClipLoss.forward` does not build logits: it calls the fused CUDA path (clipk.ops.FusedClipLoss ->
-libclipk.so).  Deviations from the reference, all deliberate:
+`ClipLoss.forward` does not build logits: it calls clipk.ops.fused_clip_loss, which runs the fused step or the general
+route of libclipk.so.  Deviations from the reference, all deliberate:
   * the loss is returned in fp32 even for pure-bf16 inputs (the reference returns bf16 there, which alone costs
     up to 2^-9 relative);
   * no per-step rank-0 prints (reference loss.py:79,110);

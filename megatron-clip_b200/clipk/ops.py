@@ -1,9 +1,9 @@
-"""Host side of the fused contrastive loss: a torch.autograd.Function over the clipk C ABI.
+"""Host side of the fused contrastive loss: two torch.autograd.Functions over the clipk C ABI.
 
 Data flow on rank r of W (b local rows, N = W*b), replacing open_CLIP/src/open_clip/loss.py:20-64, 104-140:
 
   forward   operand pass over the local rows (normalise / cast, statistics)      \
-            T_all = all-gather of the text operand rows                           |  fused step: ONE enqueue,
+            T_all = all-gather of the text operand rows                           |  _FusedStep: ONE enqueue,
             row AND column statistics of S = s * I_loc @ T_all^T  [b x N]         |  clipk_step_forward; between
             from ONE sweep over the tiles (two exact sweeps when unsafe)          |  2..8 ranks every exchange is a
             all-gather of the [3, N] column statistics                            |  pull from peer-mapped memory
@@ -11,9 +11,9 @@ Data flow on rank r of W (b local rows, N = W*b), replacing open_CLIP/src/open_c
   backward  G = alpha*(P_row-Id) + beta*(P_col-Id) tile by tile; dI_loc = c G @ T_all;   clipk_step_backward: the tiles of
             dT_partial[N, d] = c G^T @ I_loc; dT_loc = sum over ranks of their parts     dT go straight to their owners
 
-Route 2 (fp32 / fp16 arithmetic, widths that are not multiples of 64, more than 8 ranks, no symmetric memory) runs the
-same mathematics through the individual entries (clipk_fwd_both, clipk_finalize, clipk_bwd, ...) with NCCL
-all_gather_into_tensor / reduce_scatter_tensor between them.
+The general route (_GeneralRoute: fp32 / fp16 arithmetic, widths that are not multiples of 64, more than 8 ranks, no
+symmetric memory) runs the same mathematics through the individual entries (clipk_fwd_both, clipk_finalize, clipk_bwd,
+...) with NCCL all_gather_into_tensor / reduce_scatter_tensor between them.  fused_clip_loss picks the route.
 
 The [b x N] logits are never written to HBM and I_all is never gathered.  All four (local_loss,
 gather_with_grad) modes of the reference are coefficient choices of this one pipeline (SURVEY.md App. A).
@@ -43,7 +43,7 @@ def _round_up(x, m):
 
 
 def set_backend_for_testing(backend):
-    """Install an object exposing fwd_stats/fwd_both/finalize/bwd/cast/prepare (tests only; None restores CUDA)."""
+    """Install an object with the methods of CudaBackend, peer_context included (tests only; None restores CUDA)."""
     global _TEST_BACKEND
     _TEST_BACKEND = backend
 
@@ -185,6 +185,11 @@ class CudaBackend:
         return dX, dY
 
     # ---- the whole step in two enqueues (clipk_step_forward / clipk_step_backward)
+    def peer_context(self, b, d, rank, world, group):
+        """PeerContext of the fused step on 2..8 ranks, or None: the general route takes the call (see _peer_context).
+        On the current device, the one the library enqueues the step on."""
+        return _peer_context(b, d, rank, world, group, torch.device("cuda", torch.cuda.current_device()))
+
     def _c_step(self, st: "StepDesc"):
         c = st.cstruct
         if c is None:
@@ -441,7 +446,7 @@ _MAX_PEER_CONTEXTS = 4      # shapes (train batch, eval batch, ...) that get sym
 def _peer_context(b, d, rank, world, group, dev):
     """PeerContext for this shape, or None when the collectives go through NCCL instead (CLIPK_PEER=0, no symmetric
     memory on this system, more than 8 ranks, a local batch that is not a multiple of 128)."""
-    if _PEER_DISABLED[0] or os.environ.get("CLIPK_PEER", "1") == "0" or _TEST_BACKEND is not None:
+    if _PEER_DISABLED[0] or os.environ.get("CLIPK_PEER", "1") == "0":
         return None
     if dev.type != "cuda" or world < 2 or world > _lib.MAX_PEERS or b % 128 != 0:
         return None
@@ -528,114 +533,137 @@ def _row_layout_ok(x):
     return x.stride(1) == 1 and (x.stride(0) * es) % 16 == 0 and x.stride(0) >= x.shape[1] and x.data_ptr() % 16 == 0
 
 
-class FusedClipLoss(torch.autograd.Function):
-    """loss = ClipLoss(local_loss, gather_with_grad, rank, world_size).forward(I, T, s)   (loss.py:123-140).
+def _kernel_features(x):
+    """Contiguous features as the individual entries take them.  fp16 features (open_clip --precision fp16 / amp) become
+    fp32: every fp16 value is an fp32 value, so they take the split-precision fp32 path unchanged.  The kernels stream K
+    in 64-element blocks from 16-byte aligned rows, so other widths are zero-padded to the next multiple of 64: zero
+    columns change no logit, and _caller_grad drops their gradient columns."""
+    if x.dtype == torch.float16:
+        x = x.float()
+    d = _round_up(x.shape[1], _K_BLOCK)
+    return x.contiguous() if d == x.shape[1] else torch.nn.functional.pad(x, (0, d - x.shape[1]))
 
-    Two routes.  The fused step (clipk_step_forward / clipk_step_backward: one enqueue per pass, collectives over peer
-    memory) takes bf16 operands - bf16 features, or fp32 features under bf16 autocast - of a width that is a multiple
-    of 64, on one GPU or on 2..8 ranks of one NVLink domain.  Everything else (fp32 / fp16 arithmetic, other widths,
-    more ranks, no symmetric memory, local_loss without gather_with_grad on several ranks) takes the general route:
-    the individual kernel entries with NCCL collectives between them."""
+
+def _caller_grad(be, g, d_in, in_dtype):
+    """The fp32 gradient of a _kernel_features operand in the caller's width and dtype: the padding's columns dropped,
+    cast by the kernels (clipk_cast writes bf16 or fp32), fp16 rounded from fp32 at the end."""
+    if g.shape[1] != d_in:
+        g = g[:, :d_in].contiguous()
+    g = be.cast(g, torch.bfloat16 if in_dtype == torch.bfloat16 else torch.float32)
+    return g if g.dtype == in_dtype else g.to(in_dtype)
+
+
+def _mode_coefficients(b, world, local_loss, gather_with_grad):
+    """(loss_div, grad_coef, grad_split) of a (local_loss, gather_with_grad) mode, SURVEY App. A: the loss divides by 2b
+    on one rank and in the local modes, else by 2N; c = 1/(2b) there and for global+gather_with_grad, else 1/(2N).
+    Split, loss.py:53-56 with local_loss: the gathered tensors carry no gradient, so dI sees only the image->text softmax
+    and dT only the text->image one."""
+    N = world * b
+    local = world == 1 or local_loss
+    loss_div = 2.0 * b if local else 2.0 * N
+    grad_coef = 1.0 / (2.0 * b) if (local or gather_with_grad) else 1.0 / (2.0 * N)
+    return loss_div, grad_coef, world > 1 and bool(local_loss) and not gather_with_grad
+
+
+class _FusedStep(torch.autograd.Function):
+    """The fused step: clipk_step_forward / clipk_step_backward, one enqueue per pass, on bf16 operands of a width that
+    is a multiple of 64.  On 2..8 ranks every exchange is a pull from the peer-mapped memory of `peer` (PeerContext).
+    With `normalize` the operand pass L2-normalises the features and the gradient pass applies the Jacobian."""
 
     @staticmethod
-    def forward(ctx, image_features, text_features, logit_scale, local_loss, gather_with_grad, rank, world_size,
-                group, normalize=False, eps=1e-12):
+    def forward(ctx, image_features, text_features, logit_scale, local_loss, gather_with_grad, rank, world_size, group,
+                peer, normalize, eps):
         be = _backend()
-        if image_features.dim() != 2 or image_features.shape != text_features.shape:
-            raise ValueError("image_features and text_features must both be [batch, dim]")
-        if image_features.dtype != text_features.dtype:
-            raise TypeError("image_features and text_features must have the same dtype")
+        b, d = image_features.shape
+        W = int(world_size)
+        N = W * b
+        dev = image_features.device
+        in_dtype = image_features.dtype
+        want_feat = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
+        img, txt = image_features.detach(), text_features.detach()
+        if not _row_layout_ok(img):
+            img = img.contiguous()
+        if not _row_layout_ok(txt):
+            txt = txt.contiguous()
+        st = StepDesc()
+        st.rows, st.cols, st.d, st.world, st.rank, st.group = b, N, d, W, rank, group
+        st.normalize, st.eps = bool(normalize), float(eps)
+        st.image, st.text = img, txt
+        st.scale = logit_scale.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
+        st.loss_div, st.grad_coef, st.grad_split = _mode_coefficients(b, W, local_loss, gather_with_grad)
+        produced = st.normalize or in_dtype != torch.bfloat16
+        # one fp32 allocation for everything the backward reads: lse_row | lse_col | scalars | statistics | inv norms
+        n_f = b + N + 16 + _lib.STAT_WORDS * W + (2 * b if st.normalize else 0)
+        fbuf = torch.empty(n_f, dtype=torch.float32, device=dev)
+        st.lse_row, st.lse_col = fbuf[:b], fbuf[b:b + N]
+        st.scal = fbuf[b + N:b + N + 16]
+        o = b + N + 16
+        st.stats = fbuf[o:o + _lib.STAT_WORDS * W]
+        o += _lib.STAT_WORDS * W
+        if st.normalize:
+            st.inv_x, st.inv_y = fbuf[o:o + b], fbuf[o + b:o + 2 * b]
+            o += 2 * b
+        if want_feat and W > 1:
+            # fp16 copies of the operands for the gradient GEMMs: made in the forward, under the wait for the
+            # peers' column statistics
+            st.g16 = torch.empty((b + N) * d * 2 + 256, dtype=torch.uint8, device=dev)
+        st.x_op = torch.empty(b, d, dtype=torch.bfloat16, device=dev) if produced else img
+        st.y_all = torch.empty(N, d, dtype=torch.bfloat16, device=dev) if (produced or W > 1) else txt
+        st.ws = _step_workspace(be, b, N, d, W, dev)
+        st.peer = peer
+        be.step_forward(st)
+        _LAST_STEP_STATS[0] = st.stats       # tests / bench: word 5 of a rank's row tells which forward ran
+        pair = st.scal[4:6]
+        if W > 1 and not local_loss:
+            # the global (local_loss=False) loss is the same N x N problem on every rank: sum of the ranks' parts
+            dist.all_reduce(pair, op=dist.ReduceOp.SUM, group=group)
+        ctx.step = st
+        ctx.in_dtype = in_dtype
+        ctx.scale_dtype, ctx.scale_shape = logit_scale.dtype, logit_scale.shape
+        # the inputs themselves are saved so that autograd notices an in-place change before the backward reads them
+        ctx.save_for_backward(image_features, text_features)
+        # a 0-dim view into this evaluation's own state tensor (nothing else reads that word again): no copy kernel
+        return st.scal[4]
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out):
+        _ = ctx.saved_tensors            # raises if the features were modified in place since the forward
+        st = ctx.step
+        dev = st.scale.device
+        want_feat = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
+        want_scale = ctx.needs_input_grad[2]
+        st.grad_out = grad_out.detach().to(torch.float32).reshape(1).contiguous()
+        st.out_dtype = torch.bfloat16 if ctx.in_dtype == torch.bfloat16 else torch.float32
+        if want_feat:
+            st.d_image = torch.empty(st.rows, st.d, dtype=st.out_dtype, device=dev)
+            st.d_text = torch.empty(st.rows, st.d, dtype=st.out_dtype, device=dev)
+        st.d_scale = torch.empty(1, dtype=torch.float32, device=dev) if want_scale else None
+        if want_feat or want_scale or st.peer is not None:      # with peers every rank takes part in the barrier
+            _backend().step_backward(st)
+        d_scale = st.d_scale.reshape(ctx.scale_shape).to(ctx.scale_dtype) if want_scale else None
+        ctx.step = None
+        return st.d_image, st.d_text, d_scale, None, None, None, None, None, None, None, None
+
+
+class _GeneralRoute(torch.autograd.Function):
+    """Every call the fused step does not take: the individual kernel entries (clipk_fwd_both, clipk_finalize,
+    clipk_bwd, ...) with NCCL all_gather_into_tensor / reduce_scatter_tensor between them."""
+
+    @staticmethod
+    def forward(ctx, image_features, text_features, logit_scale, local_loss, gather_with_grad, rank, world_size, group):
+        be = _backend()
         b, d_in = image_features.shape
         W = int(world_size)
         N = W * b
         dev = image_features.device
         in_dtype = image_features.dtype
-        if in_dtype not in _FEATURE_DTYPES:
-            raise TypeError(f"clipk: unsupported feature dtype {in_dtype} (bf16, fp16 and fp32 only)")
         scale = logit_scale.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
-        ctx.scale_is_param = isinstance(logit_scale, torch.Tensor)
-        ctx.scale_dtype = logit_scale.dtype
-        ctx.scale_shape = logit_scale.shape
-        want_feat = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
-
-        # ---- route 1: the fused step
-        bf16_operands = in_dtype == torch.bfloat16 or (in_dtype == torch.float32 and _autocast_bf16(dev))
-        fused = bf16_operands and d_in % _K_BLOCK == 0 and (dev.type == "cuda" or _TEST_BACKEND is not None) and \
-            hasattr(be, "step_forward")
-        peer = None
-        if fused and W > 1:
-            peer = _TEST_BACKEND.peer_context(b, d_in, rank, W, group) if _TEST_BACKEND is not None else \
-                _peer_context(b, d_in, rank, W, group, dev)
-            fused = peer is not None
-        if fused:
-            img, txt = image_features.detach(), text_features.detach()
-            if not _row_layout_ok(img):
-                img = img.contiguous()
-            if not _row_layout_ok(txt):
-                txt = txt.contiguous()
-            st = StepDesc()
-            st.rows, st.cols, st.d, st.world, st.rank, st.group = b, N, d_in, W, rank, group
-            st.normalize, st.eps = bool(normalize), float(eps)
-            st.image, st.text, st.scale = img, txt, scale
-            local = (W == 1) or local_loss
-            st.loss_div = 2.0 * b if local else 2.0 * N
-            # c of SURVEY App. A: 1/(2b) for W=1, local modes and global+gather_with_grad; 1/(2N) otherwise
-            st.grad_coef = 1.0 / (2.0 * b) if (local or gather_with_grad) else 1.0 / (2.0 * N)
-            # loss.py:53-56 with local_loss: the gathered tensors carry no gradient, so dI sees only the image->text
-            # softmax and dT only the text->image one - two planes of one recompute
-            st.grad_split = W > 1 and bool(local_loss) and not gather_with_grad
-            produced = st.normalize or in_dtype != torch.bfloat16
-            # one fp32 allocation for everything the backward reads: lse_row | lse_col | scalars | statistics | inv norms
-            n_f = b + N + 16 + _lib.STAT_WORDS * W + (2 * b if st.normalize else 0)
-            fbuf = torch.empty(n_f, dtype=torch.float32, device=dev)
-            st.lse_row, st.lse_col = fbuf[:b], fbuf[b:b + N]
-            st.scal = fbuf[b + N:b + N + 16]
-            o = b + N + 16
-            st.stats = fbuf[o:o + _lib.STAT_WORDS * W]
-            o += _lib.STAT_WORDS * W
-            if st.normalize:
-                st.inv_x, st.inv_y = fbuf[o:o + b], fbuf[o + b:o + 2 * b]
-                o += 2 * b
-            if want_feat and W > 1:
-                # fp16 copies of the operands for the gradient GEMMs: made in the forward, under the wait for the
-                # peers' column statistics
-                st.g16 = torch.empty((b + N) * d_in * 2 + 256, dtype=torch.uint8, device=dev)
-            st.x_op = torch.empty(b, d_in, dtype=torch.bfloat16, device=dev) if produced else img
-            st.y_all = torch.empty(N, d_in, dtype=torch.bfloat16, device=dev) if (produced or W > 1) else txt
-            st.ws = _step_workspace(be, b, N, d_in, W, dev)
-            st.peer = peer
-            be.step_forward(st)
-            _LAST_STEP_STATS[0] = st.stats       # tests / bench: word 5 of a rank's row tells which forward ran
-            pair = st.scal[4:6]
-            if W > 1 and not local_loss:
-                # the global (local_loss=False) loss is the same N x N problem on every rank: sum of the ranks' parts
-                dist.all_reduce(pair, op=dist.ReduceOp.SUM, group=group)
-            ctx.step = st
-            ctx.in_dtype = in_dtype
-            # the inputs themselves are saved so that autograd notices an in-place change before the backward reads them
-            ctx.save_for_backward(image_features, text_features)
-            ctx.fused = True
-            # a 0-dim view into this evaluation's own state tensor (nothing else reads that word again): no copy kernel
-            return st.scal[4]
-
-        # ---- route 2: individual entries + NCCL
-        ctx.fused = False
-        if normalize:
-            raise RuntimeError("clipk: internal error - the general route does not normalise (see fused_normalize_clip_loss)")
-        # under torch.autocast the reference's matmuls run in the autocast dtype (SURVEY App. B)
         feats_i, feats_t = image_features.detach(), text_features.detach()
+        # under torch.autocast the reference's matmuls run in the autocast dtype (SURVEY App. B)
         if in_dtype == torch.float32 and _autocast_bf16(dev):
             feats_i, feats_t = feats_i.to(torch.bfloat16), feats_t.to(torch.bfloat16)
-        if in_dtype == torch.float16:
-            # fp16 features (open_clip --precision fp16 / amp): every fp16 value is an fp32 value, so they take the
-            # split-precision fp32 path unchanged; gradients are rounded back to fp16 at the end
-            feats_i, feats_t = feats_i.float(), feats_t.float()
-        # the kernels stream K in 64-element blocks from 16-byte aligned rows: other widths are zero-padded to the
-        # next multiple of 64 (zero columns change no logit; their gradient columns are dropped in the backward)
-        d = _round_up(d_in, _K_BLOCK)
-        if d != d_in:
-            feats_i = torch.nn.functional.pad(feats_i, (0, d - d_in))
-            feats_t = torch.nn.functional.pad(feats_t, (0, d - d_in))
+        feats_i, feats_t = _kernel_features(feats_i), _kernel_features(feats_t)
 
         t_all = _all_gather_rows(feats_t, W, group) if W > 1 else feats_t
         X = be.prepare(feats_i)
@@ -651,61 +679,33 @@ class FusedClipLoss(torch.autograd.Function):
         # sums[0:2] -> loss, sums[2:4] -> s * dloss/ds; the global (local_loss=False) loss is the same N x N problem
         # on every rank, so both are all-reduced there.  dlogit_scale is never reduced by the loss in local mode
         # (DDP averages it later), exactly like the reference.
+        loss_div, grad_coef, grad_split = _mode_coefficients(b, W, local_loss, gather_with_grad)
         pair = sums.view(2, 2).sum(dim=1)
         if W > 1 and not local_loss:
             dist.all_reduce(pair, op=dist.ReduceOp.SUM, group=group)
-            pair = pair / (2.0 * N)
-        else:
-            pair = pair / (2.0 * b)
-        loss = pair[0]
+        pair = pair / loss_div
 
         ctx.save_for_backward(image_features, text_features, scale, lse_row, lse_col, pair)
         ctx.operands = (X, Y)
-        ctx.cfg = (b, d, W, rank, off, bool(local_loss), bool(gather_with_grad), group, in_dtype, d_in)
-        return loss.clone()
+        ctx.cfg = (W, off, grad_coef, grad_split, group, in_dtype, d_in, logit_scale.dtype, logit_scale.shape)
+        return pair[0].clone()
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, grad_out):
         be = _backend()
         go = grad_out.detach().to(torch.float32).reshape(1)
-        if ctx.fused:
-            _ = ctx.saved_tensors            # raises if the features were modified in place since the forward
-            st = ctx.step
-            dev = st.scale.device
-            want_feat = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
-            want_scale = ctx.scale_is_param and ctx.needs_input_grad[2]
-            st.grad_out = go.contiguous()
-            st.out_dtype = torch.bfloat16 if ctx.in_dtype == torch.bfloat16 else torch.float32
-            if want_feat:
-                st.d_image = torch.empty(st.rows, st.d, dtype=st.out_dtype, device=dev)
-                st.d_text = torch.empty(st.rows, st.d, dtype=st.out_dtype, device=dev)
-            st.d_scale = torch.empty(1, dtype=torch.float32, device=dev) if want_scale else None
-            if want_feat or want_scale or st.peer is not None:      # with peers every rank takes part in the barrier
-                be.step_backward(st)
-            d_scale = st.d_scale.reshape(ctx.scale_shape).to(ctx.scale_dtype) if want_scale else None
-            d_image, d_text = st.d_image, st.d_text
-            ctx.step = None
-            return d_image, d_text, d_scale, None, None, None, None, None, None, None
-
         _, _, scale, lse_row, lse_col, pair = ctx.saved_tensors
         X, Y = ctx.operands
-        b, d, W, rank, off, local_loss, gwg, group, in_dtype, d_in = ctx.cfg
-        # dtype the kernels produce directly (clipk_cast writes bf16 or fp32)
-        k_dtype = torch.bfloat16 if in_dtype == torch.bfloat16 else torch.float32
-        N = W * b
+        W, off, grad_coef, grad_split, group, in_dtype, d_in, scale_dtype, scale_shape = ctx.cfg
         d_image = d_text = None
         if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
             Xg, Yg = be.prepare_grad(X), be.prepare_grad(Y)
-            local = (W == 1) or local_loss
-            # c of SURVEY App. A: 1/(2b) for W=1, both local modes and global+gather_with_grad; 1/(2N) otherwise
-            c_feat = 1.0 / (2.0 * b) if (local or gwg) else 1.0 / (2.0 * N)
-            gscale = (go * c_feat).contiguous()
-            if W > 1 and local_loss and not gwg:
-                # loss.py:53-56 with local_loss: gathered tensors carry no gradient, so dI sees only the image->text
-                # softmax and dT only the text->image one: one recompute with the two parts in two planes of the
-                # panel (one-plane operands), else (fp32 arithmetic: the planes are taken by [hi | lo]) two passes
-                if getattr(Xg, "dtype", None) == _lib.F16 or _TEST_BACKEND is not None:
+            gscale = (go * grad_coef).contiguous()
+            if grad_split:
+                # the two softmax parts in two planes of the panel of one recompute (one-plane operands), else (fp32
+                # arithmetic: the planes are taken by [hi | lo]) two passes
+                if Xg.dtype == _lib.F16 or _TEST_BACKEND is not None:
                     dX, dY = be.bwd(X, Y, Xg, Yg, scale, off, lse_row, lse_col, 1.0, 1.0, gscale, True, True, split=True)
                 else:
                     dX, _ = be.bwd(X, Y, Xg, Yg, scale, off, lse_row, lse_col, 1.0, 0.0, gscale, True, False)
@@ -714,34 +714,15 @@ class FusedClipLoss(torch.autograd.Function):
             else:
                 dX, dY = be.bwd(X, Y, Xg, Yg, scale, off, lse_row, lse_col, 1.0, 1.0, gscale, True, True)
                 dT = _reduce_scatter_rows(dY, W, group) if W > 1 else dY
-            if d != d_in:                         # drop the gradient columns of the zero padding
-                dX = dX[:, :d_in].contiguous()
-                dT = dT[:, :d_in].contiguous()
-            d_image = be.cast(dX, k_dtype)
-            d_text = be.cast(dT, k_dtype)
-            if k_dtype != in_dtype:               # fp16 features
-                d_image, d_text = d_image.to(in_dtype), d_text.to(in_dtype)
+            d_image, d_text = _caller_grad(be, dX, d_in, in_dtype), _caller_grad(be, dT, d_in, in_dtype)
 
         d_scale = None
-        if ctx.scale_is_param and ctx.needs_input_grad[2]:
+        if ctx.needs_input_grad[2]:
             # pair[1] = s * dloss/ds, already normalised (and all-reduced in global mode) by the forward
-            d_scale = (pair[1] * go[0] / scale[0]).reshape(ctx.scale_shape).to(ctx.scale_dtype)
-        return d_image, d_text, d_scale, None, None, None, None, None, None, None
+            d_scale = (pair[1] * go[0] / scale[0]).reshape(scale_shape).to(scale_dtype)
+        return d_image, d_text, d_scale, None, None, None, None, None
 
 
-def fused_clip_loss(image_features, text_features, logit_scale, local_loss=False, gather_with_grad=False, rank=0,
-                    world_size=1, group=None, normalize=False, eps=1e-12):
-    if not isinstance(logit_scale, torch.Tensor):
-        logit_scale = torch.tensor(float(logit_scale), dtype=torch.float32, device=image_features.device)
-    if image_features.dim() == 2 and image_features.shape[0] == 0 and image_features.shape == text_features.shape:
-        # empty batch: the reference's cross-entropy means over zero rows, i.e. NaN with empty gradients
-        # (loss.py:135-138); nothing to launch
-        return (image_features.sum() + text_features.sum()).float() * logit_scale.float() * float("nan")
-    return FusedClipLoss.apply(image_features, text_features, logit_scale, local_loss, gather_with_grad, rank,
-                               world_size, group, normalize, eps)
-
-
-# ----------------------------------------------------------------------------------------------------- opt-in: normalise + loss
 class _Normalize(torch.autograd.Function):
     """F.normalize(x, dim=-1) (open_clip/model.py:216,231) with its Jacobian, on the clipk kernels."""
 
@@ -759,12 +740,36 @@ class _Normalize(torch.autograd.Function):
         return _backend().normalize_bwd(g.to(y.dtype), y, inv, ctx.eps), None
 
 
-def _fused_step_applies(x, world_size, local_loss, gather_with_grad):
-    dev = x.device
-    return x.dim() == 2 and (x.dtype == torch.bfloat16 or (x.dtype == torch.float32 and _autocast_bf16(dev))) and \
-        x.shape[1] % _K_BLOCK == 0 and x.shape[0] > 0 and (dev.type == "cuda" or _TEST_BACKEND is not None) and \
-        (world_size == 1 or (world_size <= _lib.MAX_PEERS and x.shape[0] % 128 == 0 and
-                             os.environ.get("CLIPK_PEER", "1") != "0" and not _PEER_DISABLED[0]))
+def fused_clip_loss(image_features, text_features, logit_scale, local_loss=False, gather_with_grad=False, rank=0,
+                    world_size=1, group=None, normalize=False, eps=1e-12):
+    """loss = ClipLoss(local_loss, gather_with_grad, rank, world_size).forward(I, T, s)   (loss.py:123-140), of the
+    L2-normalised features when `normalize`.  Picks the route once, before anything is launched: the fused step for bf16
+    operands (bf16 features, or fp32 under bf16 autocast) with d % 64 == 0 on one GPU, or on several ranks when the
+    backend has a peer context for them (see _peer_context); the general route for everything else."""
+    if image_features.dim() != 2 or image_features.shape != text_features.shape:
+        raise ValueError("image_features and text_features must both be [batch, dim]")
+    if image_features.dtype != text_features.dtype:
+        raise TypeError("image_features and text_features must have the same dtype")
+    dtype, dev = image_features.dtype, image_features.device
+    if dtype not in _FEATURE_DTYPES:
+        raise TypeError(f"clipk: unsupported feature dtype {dtype} (bf16, fp16 and fp32 only)")
+    if not isinstance(logit_scale, torch.Tensor):
+        logit_scale = torch.tensor(float(logit_scale), dtype=torch.float32, device=dev)
+    b, d = image_features.shape
+    if b == 0:
+        # empty batch: the reference's cross-entropy means over zero rows, i.e. NaN with empty gradients
+        # (loss.py:135-138); nothing to launch
+        return (image_features.sum() + text_features.sum()).float() * logit_scale.float() * float("nan")
+    W = int(world_size)
+    mode = (local_loss, gather_with_grad, rank, W, group)
+    bf16_operands = dtype == torch.bfloat16 or (dtype == torch.float32 and _autocast_bf16(dev))
+    if bf16_operands and d % _K_BLOCK == 0 and (dev.type == "cuda" or _TEST_BACKEND is not None):
+        peer = _backend().peer_context(b, d, rank, W, group) if W > 1 else None
+        if W == 1 or peer is not None:
+            return _FusedStep.apply(image_features, text_features, logit_scale, *mode, peer, normalize, eps)
+    if normalize:
+        image_features, text_features = _Normalize.apply(image_features, eps), _Normalize.apply(text_features, eps)
+    return _GeneralRoute.apply(image_features, text_features, logit_scale, *mode)
 
 
 def fused_normalize_clip_loss(raw_image_features, raw_text_features, logit_scale, local_loss=False,
@@ -773,15 +778,9 @@ def fused_normalize_clip_loss(raw_image_features, raw_text_features, logit_scale
     `loss.py:123-140` computes, with gradients with respect to the raw embeddings.  Opt-in - the drop-in ClipLoss does
     not normalise, exactly like the reference's (SURVEY.md section 0, point 2).
 
-    With bf16 operands the normalisation lives in the load path of the step: the pass that produces the operands
-    (prep_kernel) normalises, rounds to bf16 and takes the statistics in one sweep over the rows, and the pass that casts
-    the gradients (finish_grad_kernel) applies the Jacobian - no standalone normalise / cast / norm kernels.  Other
-    dtypes compose the row-wise kernels of clipk_normalize_fwd / _bwd with the loss."""
-    if _fused_step_applies(raw_image_features, world_size, local_loss, gather_with_grad) and \
-            raw_image_features.shape == raw_text_features.shape and raw_image_features.dtype == raw_text_features.dtype:
-        return fused_clip_loss(raw_image_features, raw_text_features, logit_scale, local_loss, gather_with_grad, rank,
-                               world_size, group, normalize=True, eps=eps)
-    image_features = _Normalize.apply(raw_image_features, eps)
-    text_features = _Normalize.apply(raw_text_features, eps)
-    return fused_clip_loss(image_features, text_features, logit_scale, local_loss, gather_with_grad, rank, world_size,
-                           group)
+    On the fused step the normalisation lives in the load path: the pass that produces the operands (prep_kernel)
+    normalises, rounds to bf16 and takes the statistics in one sweep over the rows, and the pass that casts the gradients
+    (finish_grad_kernel) applies the Jacobian - no standalone normalise / cast / norm kernels.  The general route
+    composes the row-wise kernels of clipk_normalize_fwd / _bwd with the loss."""
+    return fused_clip_loss(raw_image_features, raw_text_features, logit_scale, local_loss, gather_with_grad, rank,
+                           world_size, group, normalize=True, eps=eps)
