@@ -210,6 +210,45 @@ size_t clipk_step_workspace_bytes(const clipk_step* step);
 int clipk_step_forward(const clipk_step* step);
 int clipk_step_backward(const clipk_step* step);
 
+/* ---- SigLipLoss: the pairwise sigmoid loss (open_clip >= 2.21, loss.py SigLipLoss) in two calls -----------------------
+ * For the b local rows x_i of rank r against all N = world * b text rows y_j (rank-major), with s = logit_scale (already
+ * exponentiated) and t = logit_bias:
+ *   l_ij = s x_i.y_j + t,  z_ij = +1 if j == diag_offset + i else -1,  loss = (1/b) sum_ij softplus(-z_ij l_ij),
+ *   g_ij = sigma(l_ij) - [j == diag_offset + i],
+ *   d_x = go (s/b) G Y [rows, d],  d_y = go (s/b) G^T X [cols, d] (the caller reduce-scatters it over the ranks),
+ *   d_scale = go (1/b) sum_ij g_ij x_i.y_j,  d_bias = go (1/b) sum_ij g_ij      (per rank, not reduced).
+ * The [rows, cols] logits are never stored.
+ *   clipk_siglip_forward   one A-resident tcgen05 sweep over the tiles (per row: sum of softplus, largest negative logit,
+ *                          positive logit) and two small merge kernels -> loss, gmax = largest |g_ij| of the block
+ *   clipk_siglip_backward  fp16 copies of X and Y; per panel of G: recompute sweep that writes fp16(g * 2^e), with 2^e
+ *                          chosen on the device from gmax so that the largest entry lands in [2^13, 2^14), and its row
+ *                          sums of g and g x.y; the two gradient GEMMs (gemm_pair_kernel); then d_scale, d_bias.
+ * Every sum is merged in a fixed order: two calls on the same inputs give bit-identical results.  bf16 operands,
+ * d % 64 == 0, rows 16-byte aligned.  The library allocates nothing and never synchronises. */
+#define CLIPK_SIGLIP_STATE_WORDS 8
+typedef struct clipk_siglip {
+    int rows, cols, d;                  /* local rows b, columns N (all ranks' text rows), embedding width (d % 64 == 0) */
+    const void* x; long long ldx;       /* [rows, d] bf16 image features, leading dimension in elements                */
+    const void* y; long long ldy;       /* [cols, d] bf16 text features of all ranks, rank-major                        */
+    const float* logit_scale;           /* device scalar s                                                              */
+    const float* logit_bias;            /* device scalar t (NULL = 0)                                                   */
+    long long diag_offset;              /* the positive of row i is column diag_offset + i (rank * rows)                */
+    float* state;                       /* CLIPK_SIGLIP_STATE_WORDS floats, written by the forward, read and extended   */
+                                        /* by the backward: [0] loss, [1] gmax, [2] largest negative logit, [3]         */
+                                        /* smallest positive logit, [4] 2^e of the G panel, [5] go * s / (b * 2^e)      */
+    /* backward only */
+    const float* grad_out;              /* device scalar go                                                             */
+    float* d_x;                         /* [rows, d] fp32, overwritten (NULL = not wanted)                              */
+    float* d_y;                         /* [cols, d] fp32, overwritten (NULL = not wanted)                              */
+    float* d_scale; float* d_bias;      /* device scalars (NULL = not wanted)                                           */
+    void* workspace; size_t workspace_bytes;        /* scratch of clipk_siglip_workspace_bytes(), 256-byte aligned;   */
+                                                    /* nothing in it lives from one call to the next                   */
+    void* stream;
+} clipk_siglip;
+size_t clipk_siglip_workspace_bytes(const clipk_siglip* p);
+int clipk_siglip_forward(const clipk_siglip* p);
+int clipk_siglip_backward(const clipk_siglip* p);
+
 /* ---- opt-in: the L2 normalisation in front of the loss (SURVEY section 8 f-1) ---------------------------------------
  * The reference normalises in the model, not in the loss (F.normalize, open_clip/model.py:216,231,277,281); these two
  * entries let a caller hand RAW embeddings to clipk.fused_normalize_clip_loss and get gradients with respect to them.

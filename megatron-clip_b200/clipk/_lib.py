@@ -73,7 +73,21 @@ class Step(ctypes.Structure):
                 ("peer", ctypes.POINTER(Peer)), ("workspace", _vp), ("workspace_bytes", _sz), ("stream", _vp)]
 
 
+SIGLIP_STATE_WORDS = 8
+
+
+class Siglip(ctypes.Structure):
+    """struct clipk_siglip (include/clipk.h)."""
+    _fields_ = [("rows", _i), ("cols", _i), ("d", _i), ("x", _vp), ("ldx", _ll), ("y", _vp), ("ldy", _ll),
+                ("logit_scale", _vp), ("logit_bias", _vp), ("diag_offset", _ll), ("state", _vp),
+                ("grad_out", _vp), ("d_x", _vp), ("d_y", _vp), ("d_scale", _vp), ("d_bias", _vp),
+                ("workspace", _vp), ("workspace_bytes", _sz), ("stream", _vp)]
+
+
 PROTOTYPES.update({
+    "clipk_siglip_workspace_bytes": (_sz, [ctypes.POINTER(Siglip)]),
+    "clipk_siglip_forward": (_i, [ctypes.POINTER(Siglip)]),
+    "clipk_siglip_backward": (_i, [ctypes.POINTER(Siglip)]),
     "clipk_bwd_panel": (_i, [_i, _i, _i, ctypes.POINTER(_ll), ctypes.POINTER(_ll)]),
     "clipk_profile_begin": (_i, [_vp]),
     "clipk_profile_end": (_i, [ctypes.c_char_p, _sz]),

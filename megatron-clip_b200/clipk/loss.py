@@ -30,20 +30,8 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import distill
-from .ops import fused_clip_loss, _all_gather_rows, _reduce_scatter_rows
-
-
-class _GatherRowsWithGrad(torch.autograd.Function):
-    """all-gather whose backward is a reduce-scatter SUM (what torch.distributed.nn.all_gather does on NCCL)."""
-
-    @staticmethod
-    def forward(ctx, x, world_size, group):
-        ctx.world_size, ctx.group = world_size, group
-        return _all_gather_rows(x, world_size, group)
-
-    @staticmethod
-    def backward(ctx, g):
-        return _reduce_scatter_rows(g, ctx.world_size, ctx.group), None, None
+from .ops import fused_clip_loss, _all_gather_rows, _GatherRowsWithGrad
+from .siglip import siglip_loss
 
 
 def gather_features(image_features, text_features, local_loss=False, gather_with_grad=False, rank=0, world_size=1,
@@ -190,8 +178,50 @@ class DistillClipLoss(ClipLoss):
         return contrastive_loss, distill_loss
 
 
+class SigLipLoss(nn.Module):
+    """open_clip's SigLipLoss (open_clip >= 2.21; not in the 2.15 reference tree): the pairwise sigmoid loss of
+    "Sigmoid Loss for Language Image Pre-Training" (Zhai et al., 2023).  forward calls clipk.siglip.siglip_loss: bf16
+    operands run on the clipk_siglip kernels without the [b, N] logits, everything else on the materialising formula.
+    The loss and the logit_scale / logit_bias gradients are per rank, as in open_clip; `bidir` only chooses open_clip's
+    communication pattern, so it changes no value here (the text rows are all-gathered with NCCL either way)."""
+
+    def __init__(self, cache_labels=False, rank=0, world_size=1, bidir=True, use_horovod=False):
+        super().__init__()
+        if use_horovod:
+            raise NotImplementedError("clipk: use_horovod=True is not supported")
+        self.cache_labels = cache_labels
+        self.rank = rank
+        self.world_size = world_size
+        self.bidir = bidir
+        self.use_horovod = use_horovod
+        self.prev_num_logits = 0
+        self.labels = {}
+        self.group = None
+
+    set_process_group = ClipLoss.set_process_group
+
+    def get_ground_truth(self, device, dtype, num_logits, negative_only=False) -> torch.Tensor:
+        """-1 everywhere, +1 on the diagonal unless negative_only (open_clip's labels of one block)."""
+        labels = -torch.ones((num_logits, num_logits), device=device, dtype=dtype)
+        if not negative_only:
+            labels = 2 * torch.eye(num_logits, device=device, dtype=dtype) + labels
+        return labels
+
+    def get_logits(self, image_features, text_features, logit_scale, logit_bias=None):
+        """Materialised logits of one block: logit_scale * I @ T^T (+ logit_bias)."""
+        logits = logit_scale * image_features @ text_features.T
+        if logit_bias is not None:
+            logits = logits + logit_bias
+        return logits
+
+    def forward(self, image_features, text_features, logit_scale, logit_bias, output_dict=False):
+        loss = siglip_loss(image_features, text_features, logit_scale, logit_bias, self.rank, self.world_size, self.group)
+        return {"contrastive_loss": loss} if output_dict else loss
+
+
 def create_loss(args):
-    """Same flag plumbing as the reference factory (factory.py:250-278); cache_labels is always on there."""
+    """Same flag plumbing as the reference factory (factory.py:250-278); cache_labels is always on there.  --siglip
+    (open_clip >= 2.21) returns SigLipLoss, checked after the distill and coca branches as open_clip does."""
     common = dict(local_loss=args.local_loss, gather_with_grad=args.gather_with_grad, cache_labels=True,
                   rank=args.rank, world_size=args.world_size, use_horovod=args.horovod)
     if getattr(args, "distill", False):
@@ -199,4 +229,6 @@ def create_loss(args):
     if "coca" in args.model.lower():
         return CoCaLoss(caption_loss_weight=args.coca_caption_loss_weight,
                         clip_loss_weight=args.coca_contrastive_loss_weight, **common)
+    if getattr(args, "siglip", False):
+        return SigLipLoss(rank=args.rank, world_size=args.world_size)
     return ClipLoss(**common)

@@ -236,6 +236,41 @@ class CudaBackend:
             c.peer = ctypes.pointer(st.cpeer)
         _lib.check(self.lib.clipk_step_backward(ctypes.byref(c)), "clipk_step_backward")
 
+    # ---- SigLipLoss (clipk_siglip_forward / clipk_siglip_backward, used by clipk/siglip.py)
+    def _c_siglip(self, X, Y, scale, bias, diag_offset, state):
+        c = _lib.Siglip()
+        c.rows, c.d = X.shape
+        c.cols = Y.shape[0]
+        c.x, c.ldx, c.y, c.ldy = X.data_ptr(), X.stride(0), Y.data_ptr(), Y.stride(0)
+        c.logit_scale, c.logit_bias = scale.data_ptr(), _ptr(bias)
+        c.diag_offset, c.state = diag_offset, state.data_ptr()
+        c.stream = self._stream()
+        ws = torch.empty(self.lib.clipk_siglip_workspace_bytes(ctypes.byref(c)), dtype=torch.uint8, device=X.device)
+        c.workspace, c.workspace_bytes = ws.data_ptr(), ws.numel()
+        return c, ws
+
+    def siglip_forward(self, X, Y, scale, bias, diag_offset):
+        """X [b, d], Y [N, d] bf16 (d % 64 == 0, unit inner stride); scale / bias: [1] fp32 device scalars (bias may be
+        None).  Returns (loss as a 0-dim view, state): the state carries what the backward needs."""
+        state = torch.zeros(_lib.SIGLIP_STATE_WORDS, dtype=torch.float32, device=X.device)
+        c, ws = self._c_siglip(X, Y, scale, bias, diag_offset, state)
+        _lib.check(self.lib.clipk_siglip_forward(ctypes.byref(c)), "clipk_siglip_forward")
+        return state[0], state
+
+    def siglip_backward(self, X, Y, scale, bias, diag_offset, state, grad_out, want_dx, want_dy, want_ds, want_dt):
+        """fp32 (d_x [b, d], d_y [N, d], d_scale [1], d_bias [1]); None where not wanted.  d_y is this rank's partial of
+        the gathered text gradient."""
+        dev = X.device
+        dX = torch.empty(X.shape, dtype=torch.float32, device=dev) if want_dx else None
+        dY = torch.empty(Y.shape, dtype=torch.float32, device=dev) if want_dy else None
+        ds = torch.empty(1, dtype=torch.float32, device=dev) if want_ds else None
+        dt = torch.empty(1, dtype=torch.float32, device=dev) if want_dt else None
+        c, ws = self._c_siglip(X, Y, scale, bias, diag_offset, state)
+        c.grad_out = grad_out.data_ptr()
+        c.d_x, c.d_y, c.d_scale, c.d_bias = _ptr(dX), _ptr(dY), _ptr(ds), _ptr(dt)
+        _lib.check(self.lib.clipk_siglip_backward(ctypes.byref(c)), "clipk_siglip_backward")
+        return dX, dY, ds, dt
+
     def normalize_fwd(self, x: torch.Tensor, eps: float):
         """y = x / max(|x|, eps) row-wise (same dtype), and the fp32 factors 1 / max(|x|, eps)."""
         if x.dtype not in (torch.bfloat16, torch.float32):
@@ -520,6 +555,19 @@ def _reduce_scatter_rows(x: torch.Tensor, world_size: int, group=None) -> torch.
     out = torch.empty((n,) + tuple(x.shape[1:]), dtype=x.dtype, device=x.device)
     dist.reduce_scatter_tensor(out, x.contiguous(), op=dist.ReduceOp.SUM, group=group)
     return out
+
+
+class _GatherRowsWithGrad(torch.autograd.Function):
+    """all-gather whose backward is a reduce-scatter SUM (what torch.distributed.nn.all_gather does on NCCL)."""
+
+    @staticmethod
+    def forward(ctx, x, world_size, group):
+        ctx.world_size, ctx.group = world_size, group
+        return _all_gather_rows(x, world_size, group)
+
+    @staticmethod
+    def backward(ctx, g):
+        return _reduce_scatter_rows(g, ctx.world_size, ctx.group), None, None
 
 
 # ----------------------------------------------------------------------------------------------------- autograd

@@ -1390,6 +1390,115 @@ int launch_fwd_sweep(const CUtensorMap& ta, const CUtensorMap& tb, const FwdArgs
     return launch_clustered("fwd_sweep_kernel", kfn, dim3(2 * n_clusters), dim3(2, 1, 1), smem, st, ta, tb, a);
 }
 
+// ---- SigLipLoss (clipk_siglip_forward / _backward) -------------------------------------------------------------------
+enum { SIG_LOSS = 0, SIG_GMAX = 1, SIG_MAXNEG = 2, SIG_MINPOS = 3, SIG_P2E = 4, SIG_OSCALE = 5 };   // state words
+// Largest G panel of the SigLIP backward: it stays L2-resident between the recompute that writes it and the two gradient
+// GEMMs that read it, and the backward's extra memory stays a small fraction of the b x N logits the formula holds.
+constexpr long long SIG_PANEL_BYTES = 64ll << 20;
+
+// Per row: the partial sums of the sweep's (part, half) slots, in part order.  Forward (max_b): out_a = sum of
+// softplus / ln 2, out_b = largest negative logit * log2(e).  Recompute: out_a (+)= sum g, out_b (+)= sum g x.y
+// (accumulate: later column panels add to the earlier ones, in panel order).
+__global__ void siglip_rows_kernel(const float* __restrict__ part_a, const float* __restrict__ part_b, int M,
+                                   const SweepGeom g, int n_clusters, int max_b, int accumulate, float* __restrict__ out_a,
+                                   float* __restrict__ out_b) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= M) return;
+    const long long total = (long long)g.m_pairs * g.n_tiles, f = (long long)(i / (2 * BM)) * g.n_tiles;
+    const int nparts = PARTS_PER_UNIT * (sweep_cluster_of(total, f + g.n_tiles - 1, n_clusters) - sweep_cluster_of(total, f, n_clusters) + 1);
+    float a = 0.f, b = max_b ? -CUDART_INF_F : 0.f;
+    for (int p = 0; p < nparts; ++p) {
+        a += part_a[(size_t)p * M + i];
+        const float v = part_b[(size_t)p * M + i];
+        b = max_b ? fmaxf(b, v) : b + v;
+    }
+    if (accumulate) { a += out_a[i]; b += out_b[i]; }
+    out_a[i] = a;
+    out_b[i] = b;
+}
+
+__device__ __forceinline__ float sig_sigmoid(float x) { return 1.f / (1.f + expf(-x)); }
+
+// One block of 1024 threads, fixed-order sums over the rows (strided per thread, then a tree).
+//   forward  (go == null): state[LOSS] = ln 2 / b * sum row_a, [MAXNEG] = max row_b * ln 2, [MINPOS] = min pos,
+//                          [GMAX] = max(sigma(MAXNEG), sigma(-MINPOS)) = the largest |g| of the block
+//   backward            : d_bias = go / b * sum row_a, d_scale = go / b * sum row_b  (either may be null)
+__global__ void __launch_bounds__(1024) siglip_reduce_kernel(const float* __restrict__ row_a, const float* __restrict__ row_b,
+                                                             const float* __restrict__ pos, int M, float* __restrict__ state,
+                                                             const float* __restrict__ go, float* d_scale, float* d_bias) {
+    __shared__ float sa[1024], sb[1024], sp[1024];
+    const int tid = threadIdx.x;
+    const bool fwd = go == nullptr;
+    float a = 0.f, b = fwd ? -CUDART_INF_F : 0.f, pm = CUDART_INF_F;
+    for (int i = tid; i < M; i += 1024) {
+        a += row_a[i];
+        if (fwd) { b = fmaxf(b, row_b[i]); pm = fminf(pm, pos[i]); }
+        else b += row_b[i];
+    }
+    sa[tid] = a; sb[tid] = b; sp[tid] = pm;
+    __syncthreads();
+    for (int w = 512; w > 0; w >>= 1) {
+        if (tid < w) {
+            sa[tid] += sa[tid + w];
+            sb[tid] = fwd ? fmaxf(sb[tid], sb[tid + w]) : sb[tid] + sb[tid + w];
+            sp[tid] = fminf(sp[tid], sp[tid + w]);
+        }
+        __syncthreads();
+    }
+    if (tid != 0) return;
+    if (fwd) {
+        const float maxneg = sb[0] * LN2, minpos = sp[0];
+        state[SIG_LOSS] = sa[0] * LN2 / float(M);
+        state[SIG_MAXNEG] = maxneg;
+        state[SIG_MINPOS] = minpos;
+        state[SIG_GMAX] = fmaxf(maxneg > -CUDART_INF_F ? sig_sigmoid(maxneg) : 0.f, sig_sigmoid(-minpos));
+    } else {
+        const float k = go[0] / float(M);
+        if (d_bias) d_bias[0] = sa[0] * k;
+        if (d_scale) d_scale[0] = sb[0] * k;
+    }
+}
+
+// The power of two of the G panel, from gmax: the largest |g| * 2^e lands in [2^13, 2^14) of fp16 (CLIP's fixed 2^14
+// would leave a well-separated batch, every |g| ~ 2e-9, in fp16 subnormals).  e <= 64 keeps go * s / (b * 2^e) times the
+// fp16 operand scales a normal fp32 number; gmax = 0 / NaN (a NaN feature) takes 2^14.
+__global__ void siglip_bwd_prep_kernel(float* __restrict__ state, const float* __restrict__ go,
+                                       const float* __restrict__ scale, int rows) {
+    const float gmax = state[SIG_GMAX];
+    int e = 14;
+    if (gmax > 0.f && gmax <= 1.f) {
+        int k = 0;
+        frexpf(gmax, &k);                  // gmax = m * 2^k, m in [0.5, 1)
+        e = 14 - k;
+        if (e > 64) e = 64;
+    }
+    state[SIG_P2E] = ldexpf(1.f, e);
+    state[SIG_OSCALE] = go[0] * scale[0] / float(rows) * ldexpf(1.f, -e);
+}
+
+template <bool ARES>
+static int launch_sig_fwd(const CUtensorMap& ta, const CUtensorMap& tb, const SigArgs& a, const SweepGeom& g, int n_clusters,
+                          cudaStream_t st) {
+    auto kfn = siglip_fwd_kernel<ARES>;
+    constexpr int smem = smem_bytes_sig_fwd(ARES);
+    static std::once_flag once;
+    static cudaError_t attr_err = cudaSuccess;
+    std::call_once(once, [&] { attr_err = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
+    if (attr_err != cudaSuccess) return fail(int(attr_err), "cudaFuncSetAttribute: %s", cudaGetErrorString(attr_err));
+    return launch_clustered("siglip_fwd_kernel", kfn, dim3(2 * n_clusters), dim3(2, 1, 1), smem, st, ta, tb, a, g);
+}
+template <bool ARES>
+static int launch_sig_grad(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc, const SigArgs& a,
+                           const SweepGeom& g, int n_clusters, cudaStream_t st) {
+    auto kfn = siglip_grad_kernel<ARES>;
+    constexpr int smem = smem_bytes_sig_grad(ARES);
+    static std::once_flag once;
+    static cudaError_t attr_err = cudaSuccess;
+    std::call_once(once, [&] { attr_err = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
+    if (attr_err != cudaSuccess) return fail(int(attr_err), "cudaFuncSetAttribute: %s", cudaGetErrorString(attr_err));
+    return launch_clustered("siglip_grad_kernel", kfn, dim3(2 * n_clusters), dim3(2, 1, 1), smem, st, ta, tb, tc, a, g);
+}
+
 }  // namespace clipk
 
 using namespace clipk;
@@ -2224,6 +2333,179 @@ int clipk_step_backward(const clipk_step* p) {
         fa.pair = p->scal + 4; fa.go = p->grad_out; fa.scale = p->logit_scale; fa.dscale = p->d_scale;
         finish_grad_kernel<<<1, 32, 0, st>>>(fa);
         count_launch("finish_grad_kernel", st);
+        CK_CUDA(cudaGetLastError());
+    }
+    return CLIPK_OK;
+}
+
+// ---- SigLipLoss (see include/clipk.h) ---------------------------------------------------------------------------------
+namespace {
+struct SigCarve {
+    size_t part_a, part_b, pos, row_a, row_b, scale_io, xg, yg, g, total;
+    long long g_bytes;
+};
+SigCarve sig_carve(int rows, int cols, int d) {
+    SigCarve c{};
+    auto take = [](size_t& off, size_t bytes) { const size_t o = off; off = size_t(round_up((long long)(off + bytes), 256)); return o; };
+    // sweep_parts_bound(n) * n <= 32768 + 2n for every row count n: the slots of the forward and of any row panel
+    const size_t parts = size_t(PARTS_PER_UNIT) * (32768 + 2 * size_t(rows)) * sizeof(float);
+    size_t off = 0;
+    c.part_a = take(off, parts);
+    c.part_b = take(off, parts);
+    c.pos = take(off, size_t(rows) * sizeof(float));
+    c.row_a = take(off, size_t(rows) * sizeof(float));
+    c.row_b = take(off, size_t(rows) * sizeof(float));
+    c.scale_io = take(off, 4 * sizeof(float));
+    c.xg = take(off, size_t(rows) * d * 2);
+    c.yg = take(off, size_t(cols) * d * 2);
+    c.g_bytes = std::min(SIG_PANEL_BYTES, round_up(rows, 2 * BM) * round_up(cols, BN) * 2);
+    c.g = take(off, size_t(c.g_bytes));
+    c.total = off;
+    return c;
+}
+int sig_check(const clipk_siglip* p) {
+    if (!p) return fail(CLIPK_EINVAL, "null argument");
+    if (p->rows <= 0 || p->cols <= 0 || p->d <= 0) return fail(CLIPK_EINVAL, "rows, cols and d must be positive");
+    if (p->d % BK != 0) return fail(CLIPK_EUNSUPPORTED, "d = %d is not a multiple of 64", p->d);
+    if (p->diag_offset < 0 || p->diag_offset + p->rows > p->cols) return fail(CLIPK_EINVAL, "the positives must be columns of the block");
+    if (!p->x || !p->y || !p->logit_scale || !p->state || !p->workspace) return fail(CLIPK_EINVAL, "null pointer argument");
+    if (p->ldx < p->d || p->ldy < p->d || (p->ldx * 2) % 16 != 0 || (p->ldy * 2) % 16 != 0 ||
+        (reinterpret_cast<uintptr_t>(p->x) & 15) != 0 || (reinterpret_cast<uintptr_t>(p->y) & 15) != 0)
+        return fail(CLIPK_EINVAL, "feature rows must be 16-byte aligned and at least d wide");
+    if ((reinterpret_cast<uintptr_t>(p->workspace) & 255) != 0) return fail(CLIPK_EINVAL, "workspace must be 256-byte aligned");
+    if (p->workspace_bytes < sig_carve(p->rows, p->cols, p->d).total) return fail(CLIPK_EWORKSPACE, "workspace too small");
+    return CLIPK_OK;
+}
+}  // namespace
+
+size_t clipk_siglip_workspace_bytes(const clipk_siglip* p) {
+    if (!p || p->rows <= 0 || p->cols <= 0 || p->d <= 0) return 0;
+    return sig_carve(p->rows, p->cols, p->d).total;
+}
+
+int clipk_siglip_forward(const clipk_siglip* p) {
+    int rc;
+    if ((rc = sig_check(p))) return rc;
+    DevInfo di;
+    if ((rc = device_info(&di))) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(p->stream);
+    const int rows = p->rows, cols = p->cols, d = p->d;
+    const SigCarve cv = sig_carve(rows, cols, d);
+    char* ws = static_cast<char*>(p->workspace);
+    CUtensorMap ta, tb;
+    if ((rc = tmap_kmajor(&ta, p->x, rows, d, p->ldx, BM))) return rc;
+    if ((rc = tmap_kmajor(&tb, p->y, cols, d, p->ldy, BN / 2))) return rc;
+    SweepGeom g{};
+    g.num_kb = d / BK; g.n_tiles = cdiv(cols, BN); g.m_pairs = cdiv(rows, 2 * BM);
+    const int nc = int(std::min<long long>(di.sms / 2, (long long)g.m_pairs * g.n_tiles));
+    SigArgs a{};
+    a.M = rows; a.N = cols; a.scale = p->logit_scale; a.bias = p->logit_bias; a.diag_offset = p->diag_offset;
+    a.part_a = reinterpret_cast<float*>(ws + cv.part_a); a.part_b = reinterpret_cast<float*>(ws + cv.part_b);
+    a.pos = reinterpret_cast<float*>(ws + cv.pos);
+    rc = g.num_kb <= ARES_KB ? launch_sig_fwd<true>(ta, tb, a, g, nc, st) : launch_sig_fwd<false>(ta, tb, a, g, nc, st);
+    if (rc) return rc;
+    float* row_a = reinterpret_cast<float*>(ws + cv.row_a);
+    float* row_b = reinterpret_cast<float*>(ws + cv.row_b);
+    siglip_rows_kernel<<<cdiv(rows, 256), 256, 0, st>>>(a.part_a, a.part_b, rows, g, nc, 1, 0, row_a, row_b);
+    count_launch("siglip_rows_kernel", st);
+    siglip_reduce_kernel<<<1, 1024, 0, st>>>(row_a, row_b, a.pos, rows, p->state, nullptr, nullptr, nullptr);
+    count_launch("siglip_reduce_kernel", st);
+    CK_CUDA(cudaGetLastError());
+    return CLIPK_OK;
+}
+
+int clipk_siglip_backward(const clipk_siglip* p) {
+    int rc;
+    if ((rc = sig_check(p))) return rc;
+    if (!p->grad_out) return fail(CLIPK_EINVAL, "null grad_out");
+    const bool want_feat = p->d_x || p->d_y;
+    if (!want_feat && !p->d_scale && !p->d_bias) return CLIPK_OK;
+    DevInfo di;
+    if ((rc = device_info(&di))) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(p->stream);
+    const int rows = p->rows, cols = p->cols, d = p->d;
+    const SigCarve cv = sig_carve(rows, cols, d);
+    char* ws = static_cast<char*>(p->workspace);
+    float* state = p->state;
+    siglip_bwd_prep_kernel<<<1, 1, 0, st>>>(state, p->grad_out, p->logit_scale, rows);
+    count_launch("siglip_bwd_prep_kernel", st);
+    CK_CUDA(cudaGetLastError());
+    // exact fp16 copies of both operands for the gradient GEMMs (fp16 x fp16: the G panel needs fp16's mantissa)
+    __half* Xg = reinterpret_cast<__half*>(ws + cv.xg);
+    __half* Yg = reinterpret_cast<__half*>(ws + cv.yg);
+    float* scale_io = reinterpret_cast<float*>(ws + cv.scale_io);     // [0..1] of Xg, [2..3] of Yg; [1], [3] = inv_scale
+    if (want_feat) {
+        if ((rc = to_f16_impl(p->x, CLIPK_BF16, rows, d, p->ldx, Xg, 1, d, scale_io, nullptr, p->stream))) return rc;
+        if ((rc = to_f16_impl(p->y, CLIPK_BF16, cols, d, p->ldy, Yg, 1, d, scale_io + 2, nullptr, p->stream))) return rc;
+    }
+    long long rp, cp;
+    choose_panel(rows, cols, d, 1, di.sms, cv.g_bytes, &rp, &cp);
+    if (round_up(rp, 2 * BM) * cp * 2 > cv.g_bytes) return fail(CLIPK_EWORKSPACE, "panel does not fit the workspace");
+    __half* G = reinterpret_cast<__half*>(ws + cv.g);
+    float* part_a = reinterpret_cast<float*>(ws + cv.part_a);
+    float* part_b = reinterpret_cast<float*>(ws + cv.part_b);
+    float* row_a = reinterpret_cast<float*>(ws + cv.row_a);
+    float* row_b = reinterpret_cast<float*>(ws + cv.row_b);
+    const char* Xb = static_cast<const char*>(p->x);
+    const char* Yb = static_cast<const char*>(p->y);
+    const int nt = cdiv(d, BN), num_kb = d / BK;
+    PeerOut no_peers;
+    memset(&no_peers, 0, sizeof(no_peers));
+    for (long long r0 = 0; r0 < rows; r0 += rp) {
+        const int nr = int(std::min<long long>(rows - r0, rp));
+        for (long long c0 = 0; c0 < cols; c0 += cp) {
+            const int nc = int(std::min<long long>(cols - c0, cp));
+            // ---- recompute the panel: G = fp16(g * 2^e), row sums of g and g x.y
+            CUtensorMap ta, tb, tc;
+            if ((rc = tmap_kmajor(&ta, Xb + r0 * p->ldx * 2, nr, d, p->ldx, BM))) return rc;
+            if ((rc = tmap_kmajor(&tb, Yb + c0 * p->ldy * 2, nc, d, p->ldy, BN / 2))) return rc;
+            if ((rc = tmap_g_store_dense32(&tc, G, round_up(nr, 2 * BM), cp, cp))) return rc;
+            SigArgs a{};
+            a.M = nr; a.N = nc; a.scale = p->logit_scale; a.bias = p->logit_bias; a.diag_offset = p->diag_offset + r0 - c0;
+            a.part_a = part_a; a.part_b = part_b; a.p2e = state + SIG_P2E;
+            SweepGeom g{};
+            g.num_kb = num_kb; g.n_tiles = cdiv(nc, BN); g.m_pairs = cdiv(nr, 2 * BM);
+            const int ncl = int(std::min<long long>(di.sms / 2, (long long)g.m_pairs * g.n_tiles));
+            rc = num_kb <= ARES_KB ? launch_sig_grad<true>(ta, tb, tc, a, g, ncl, st) : launch_sig_grad<false>(ta, tb, tc, a, g, ncl, st);
+            if (rc) return rc;
+            siglip_rows_kernel<<<cdiv(nr, 256), 256, 0, st>>>(part_a, part_b, nr, g, ncl, 0, c0 > 0 ? 1 : 0, row_a + r0, row_b + r0);
+            count_launch("siglip_rows_kernel", st);
+            CK_CUDA(cudaGetLastError());
+            if (!want_feat) continue;
+            // ---- job 0: d_x[r0:r0+nr] (+)= G Yg[c0:c0+nc];  job 1: d_y[c0:c0+nc] (+)= G^T Xg[r0:r0+nr];
+            //      scaled by go * s / (b * 2^e) (state) and the fp16 copy's inverse scale
+            CUtensorMap ta0, tb0, tc0, ta1, tb1, tc1;
+            KArgs a0{}, a1{};
+            int jobs0 = 0, jobs1 = 0;
+            if (p->d_x) {
+                if ((rc = tmap_kmajor(&ta0, G, nr, nc, cp, BM))) return rc;
+                if ((rc = tmap_mnmajor(&tb0, Yg + c0 * d, d, nc, d))) return rc;
+                if ((rc = tmap_out_f32(&tc0, p->d_x + r0 * d, nr, d, d))) return rc;
+                a0.M = nr; a0.N = d; a0.n_tiles = nt; a0.tiles_per_unit = 1; a0.a_mn = 0; a0.b_mn = 1;
+                set_segments(a0, 1, nc, cp, d);
+                a0.out = p->d_x + r0 * d; a0.ldo = d; a0.accumulate = c0 > 0 ? 1 : 0;
+                a0.oscale0 = state + SIG_OSCALE; a0.oscale1 = scale_io + 3; a0.oconst = 1.f;
+                jobs0 = cdiv(nr, 2 * BM) * nt;
+            }
+            if (p->d_y) {
+                if ((rc = tmap_mnmajor(&ta1, G, nc, nr, cp))) return rc;
+                if ((rc = tmap_mnmajor(&tb1, Xg + r0 * d, d, nr, d))) return rc;
+                if ((rc = tmap_out_f32(&tc1, p->d_y + c0 * d, nc, d, d))) return rc;
+                a1.M = nc; a1.N = d; a1.n_tiles = nt; a1.tiles_per_unit = 1; a1.a_mn = 1; a1.b_mn = 1;
+                set_segments(a1, 1, nr, cp, d);
+                a1.out = p->d_y + c0 * d; a1.ldo = d; a1.accumulate = r0 > 0 ? 1 : 0;
+                a1.oscale0 = state + SIG_OSCALE; a1.oscale1 = scale_io + 1; a1.oconst = 1.f;
+                jobs1 = cdiv(nc, 2 * BM) * nt;
+            }
+            if (p->d_x && p->d_y) rc = launch_pair(ta0, tb0, tc0, a0, jobs0, ta1, tb1, tc1, a1, jobs1, no_peers, st);
+            else if (p->d_x) rc = launch_gemm<MODE_OUT, 1>(ta0, tb0, tc0, a0, nt, cdiv(nr, 2 * BM), st);
+            else rc = launch_gemm<MODE_OUT, 1>(ta1, tb1, tc1, a1, nt, cdiv(nc, 2 * BM), st);
+            if (rc) return rc;
+        }
+    }
+    if (p->d_scale || p->d_bias) {
+        siglip_reduce_kernel<<<1, 1024, 0, st>>>(row_a, row_b, nullptr, rows, state, p->grad_out, p->d_scale, p->d_bias);
+        count_launch("siglip_reduce_kernel", st);
         CK_CUDA(cudaGetLastError());
     }
     return CLIPK_OK;

@@ -1228,4 +1228,293 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant
     cta_teardown(c);
 }
 
+// ---------------------------------------------------------------------------------------------------- SigLIP
+// Pairwise sigmoid loss (open_clip's SigLipLoss) over the tiles of S = X Y^T:
+//   l_ij = s x_i.y_j + t,  z_ij = +1 at the positive (column diag_offset + i), -1 elsewhere,
+//   loss = (1/b) sum_ij softplus(-z_ij l_ij),   g_ij = sigma(l_ij) - [j is the positive].
+// Every element is independent: no row or column log-sum-exp, no shared reference, no column statistics.  Both kernels
+// are the A-resident persistent sweep of the ClipLoss forward (sweep_produce / sweep_mma / SweepWalk) with an epilogue
+// of their own, one thread per row and 128-column half (the tcgen05.ld 32x32b layout).  Per (part, half, row) they
+// write plain partial sums that small kernels merge in a fixed order: the results are bit-reproducible, no atomics.
+struct SigArgs {
+    int M, N;                  // rows (b) and columns of this call's block
+    const float* scale;        // device scalar s (already exponentiated)
+    const float* bias;         // device scalar t; null = 0
+    long long diag_offset;     // the positive of row i is column diag_offset + i
+    float* part_a;             // [parts][M]  forward: sum softplus(-z l) / ln 2      recompute: sum g
+    float* part_b;             // [parts][M]  forward: max negative l * log2(e)       recompute: sum g * x.y
+    float* pos;                // [M] forward: positive logit (natural units)
+    const float* p2e;          // recompute: device scalar 2^e, the power of two the fp16 G panel carries
+};
+constexpr int SIG_GRAD_STAGES_STREAM = 6;        // B (and A) stages of the recompute when K > 512: same smem as ARES
+__host__ __device__ constexpr int smem_bytes_sig_fwd(bool ares) {
+    return 1024 + (ares ? ARES_KB : FWD_STAGES) * A_STAGE_BYTES + FWD_STAGES * B_STAGE_BYTES + 256 + MISC_BYTES;
+}
+__host__ __device__ constexpr int sig_grad_stages(bool ares) { return ares ? GRAD_SWEEP_STAGES : SIG_GRAD_STAGES_STREAM; }
+__host__ __device__ constexpr int smem_bytes_sig_grad(bool ares) {
+    return 1024 + (ares ? ARES_KB : SIG_GRAD_STAGES_STREAM) * A_STAGE_BYTES + sig_grad_stages(ares) * B_STAGE_BYTES +
+           GRAD_SWEEP_STG + 256 + MISC_BYTES;
+}
+
+// log2(1 + e) for e in [0, 1], on the FMA pipe: e * P(e) with P a degree-8 fit of log2(1 + e) / e at Chebyshev nodes.
+// Relative error <= 2e-7 in fp32 over every normal e, so small terms keep their value: lg2(1 + e) would round 1 + e
+// to 1 and drop every term below 2^-24, and a well-separated batch's loss is a sum of N such terms per row.
+__device__ __forceinline__ float sig_log2_1p(float e) {
+    float p = 7.395402063e-03f;
+    p = fmaf(p, e, -4.194501042e-02f);
+    p = fmaf(p, e, 1.118320748e-01f);
+    p = fmaf(p, e, -1.962389499e-01f);
+    p = fmaf(p, e, 2.752211988e-01f);
+    p = fmaf(p, e, -3.582990766e-01f);
+    p = fmaf(p, e, 4.806788862e-01f);
+    p = fmaf(p, e, -7.213395238e-01f);
+    p = fmaf(p, e, 1.442695022e+00f);
+    return p * e;
+}
+__device__ __forceinline__ float sig_rcp(float x) {
+    float y;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+
+// 32 columns of one row of the forward, log2 units: with u = -z l log2(e),
+//   softplus(-z l) / ln 2 = max(u, 0) + log2(1 + 2^-|u|)
+// ONE MUFU op per element (the ex2; 2^-|u| never overflows, and terms down to 2^-126 stay normal), the log on the FMA
+// pipe.  EDGE: the chunk may hold the row's positive, or columns >= N (read as zeros by TMA, masked here).
+template <bool EDGE>
+__device__ __forceinline__ void sig_fwd_chunk(const uint32_t (&r)[32], float sc2, float t2, int col0, int ncols,
+                                              long long dcol, float (&acc)[4], float& mneg, float& pos_raw, bool& have_pos) {
+    const int didx = (EDGE && dcol >= col0 && dcol < (long long)col0 + 32) ? int(dcol - col0) : -1;
+#pragma unroll
+    for (int k = 0; k < 32; ++k) {
+        const float v = fmaf(__uint_as_float(r[k]), sc2, t2);      // l * log2(e)
+        const bool is_pos = EDGE && k == didx;
+        const bool inside = !EDGE || col0 + k < ncols;
+        const float u = is_pos ? -v : v;
+        float sp = fmaxf(u, 0.f) + sig_log2_1p(ptx::ex2(-fabsf(u)));
+        if (EDGE) {
+            if (!inside) sp = 0.f;
+            if (is_pos) { pos_raw = __uint_as_float(r[k]); have_pos = true; }
+        }
+        acc[k & 3] += sp;
+        if (!is_pos && inside) mneg = fmaxf(mneg, v);
+    }
+}
+
+// One unit (a run of column tiles of one 128-row block) of the forward epilogue; writes the row's partial sums of the unit
+// into slot (part, half).  Same accumulator hand-off as epilogue_unit.
+__device__ __forceinline__ void sig_fwd_epilogue_unit(const Cta& c, Pipe& p, const SigArgs& args, int m_blk, int part, int t0,
+                                                      int t1) {
+    const int warp = c.warp, lane = c.lane;
+    const int q = warp & 3, half = (warp - 2) >> 2;
+    const int row = m_blk * BM + q * 32 + lane;
+    const long long dcol = args.diag_offset + row;
+    const float s = __ldg(args.scale), t = args.bias ? __ldg(args.bias) : 0.f;
+    const float sc2 = s * LOG2E, t2 = t * LOG2E;
+    const int ncols = args.N;
+    const long long d_lo = args.diag_offset + (long long)m_blk * BM;
+    float acc[4] = {0.f, 0.f, 0.f, 0.f}, mneg = -CUDART_INF_F, pos_raw = 0.f;
+    bool have_pos = false;
+    for (int tt = t0; tt < t1; ++tt, ++p.it) {
+        const int a = p.it & 1;
+        const uint32_t aph = (p.it >> 1) & 1;
+        const int n0 = tt * BN;
+        const int colh = n0 + half * (BN / 2);
+        // edge tile: contains positives of this CTA's rows, or columns beyond N
+        const bool edge = ((d_lo + BM - 1 >= n0) && (d_lo < (long long)n0 + BN)) || (n0 + BN > ncols);
+        ptx::mbar_wait(c.bar_tfull + 8 * a, aph);
+        ptx::tc_fence_after();
+        const uint32_t taddr = c.tmem_base + a * BN + half * (BN / 2) + (uint32_t(q * 32) << 16);
+        auto process = [&](const uint32_t (&r)[32], int cidx) {
+            const int col0 = colh + cidx * 32;
+            if (edge) sig_fwd_chunk<true>(r, sc2, t2, col0, ncols, dcol, acc, mneg, pos_raw, have_pos);
+            else sig_fwd_chunk<false>(r, sc2, t2, col0, ncols, dcol, acc, mneg, pos_raw, have_pos);
+        };
+        uint32_t ra[32], rb[32];
+        ptx::tmem_ld_32x32(taddr, ra);
+        ptx::tmem_ld_wait();
+        ptx::tmem_ld_32x32(taddr + 32, rb);
+        process(ra, 0);
+        ptx::tmem_ld_wait();
+        ptx::tmem_ld_32x32(taddr + 64, ra);
+        process(rb, 1);
+        ptx::tmem_ld_wait();
+        ptx::tmem_ld_32x32(taddr + 96, rb);
+        process(ra, 2);
+        ptx::tmem_ld_wait();
+        ptx::tc_fence_before();
+        __syncwarp();
+        if (lane == 0) ptx::mbar_arrive_leader(c.bar_tempty + 8 * a);
+        process(rb, 3);
+    }
+    if (row < args.M) {
+        const size_t slot = (size_t)(part * PARTS_PER_UNIT + half) * args.M + row;
+        args.part_a[slot] = (acc[0] + acc[1]) + (acc[2] + acc[3]);
+        args.part_b[slot] = mneg;
+        if (have_pos) args.pos[row] = fmaf(pos_raw, s, t);
+    }
+}
+
+template <bool ARES>
+__global__ void __launch_bounds__(NUM_THREADS, 1)
+siglip_fwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const SigArgs args,
+                  const SweepGeom geom) {
+    constexpr int STAGES = FWD_STAGES;
+    const Cta c = cta_setup<STAGES, 0, (ARES ? ARES_KB : STAGES) * A_STAGE_BYTES>();
+    const int cluster = blockIdx.x >> 1, n_clusters = gridDim.x >> 1;
+    Pipe p;
+    if (c.warp == 0) {
+        if (c.lane == 0) {
+            ptx::prefetch_tmap(&tmA);
+            ptx::prefetch_tmap(&tmB);
+            sweep_produce<STAGES, ARES>(c, p, &tmA, &tmB, geom, cluster, n_clusters);
+        }
+    } else if (c.warp == 1) {
+        if (c.lane == 0 && c.leader) sweep_mma<STAGES, 0, ARES>(c, p, geom, cluster, n_clusters);
+    } else {
+        const long long total = (long long)geom.m_pairs * geom.n_tiles;
+        SweepWalk w(geom, cluster, n_clusters);
+        SweepUnit un;
+        while (w.next(un)) {
+            const int part = cluster - sweep_cluster_of(total, (long long)un.m_pair * geom.n_tiles, n_clusters);
+            sig_fwd_epilogue_unit(c, p, args, 2 * un.m_pair + int(c.cta_rank), part, un.t0, un.t1);
+        }
+    }
+    cta_teardown(c);
+}
+
+// 16 columns of one row of the recompute: g = sigma(l) - [positive], times 2^e, into g[16] (fp32, still to be packed).
+// With e = exp(-|l|) (ex2) and r = 1 / (1 + e) (rcp) - TWO MUFU ops per element:
+//   sigma(l) = r for l >= 0, e * r for l < 0     (never overflows: e <= 1; no 1 - x cancellation)
+//   at the positive g = -sigma(-l), not sigma(l) - 1: a well-classified positive (l = 20) keeps g = -2e-9 instead of
+//   the 0 or 2^-24 multiples sigma(l) - 1 gives in fp32.
+// The row sums of g and g * x.y (dlogit_bias, dlogit_scale) are taken from the unscaled fp32 values.
+template <bool EDGE>
+__device__ __forceinline__ void sig_grad16(const uint32_t (&r)[16], float sc2, float t2, float p2e, int col0, int ncols,
+                                           long long dcol, bool row_ok, float& sg, float& sgx, float (&g)[16]) {
+    const int didx = (EDGE && dcol >= col0 && dcol < (long long)col0 + 16) ? int(dcol - col0) : -1;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+        const float xy = __uint_as_float(r[k]);
+        const float v = fmaf(xy, sc2, t2);                 // l * log2(e)
+        const float e = ptx::ex2(-fabsf(v));
+        const float big = sig_rcp(1.f + e), small = e * big;
+        float gk = v >= 0.f ? big : small;                 // NaN logits take `small` = NaN
+        if (EDGE) {
+            if (k == didx) gk = -(v >= 0.f ? small : big);
+            if (!row_ok || col0 + k >= ncols) gk = 0.f;
+        }
+        sg += gk;
+        sgx = fmaf(gk, xy, sgx);
+        g[k] = gk * p2e;
+    }
+}
+
+// One unit of the recompute epilogue: the G tile leaves through the same half-size SWIZZLE_64B staging and TMA stores as
+// grad_epilogue_unit<false, 1>; the row sums of the unit go to slot (part, half).
+__device__ __forceinline__ void sig_grad_epilogue_unit(const Cta& c, Pipe& p, const CUtensorMap* tmC, const SigArgs& args,
+                                                       int m_blk, int part, int t0, int t1) {
+    const int warp = c.warp, lane = c.lane;
+    const int q = warp & 3, half = (warp - 2) >> 2;
+    const int row = m_blk * BM + q * 32 + lane;
+    const bool row_ok = row < args.M;
+    const long long dcol = args.diag_offset + row;
+    const float sc2 = __ldg(args.scale) * LOG2E, t2 = (args.bias ? __ldg(args.bias) : 0.f) * LOG2E;
+    const float p2e = __ldg(args.p2e);
+    const int ncols = args.N;
+    const int c_row_off = m_blk * BM + q * 32;
+    const long long d_lo = args.diag_offset + (long long)m_blk * BM;
+    const bool row_edge = (m_blk + 1) * BM > args.M;
+    const uint32_t stg0 = c.sStg + (warp - 2) * STG_BYTES;
+    float sg = 0.f, sgx = 0.f;
+    for (int tt = t0; tt < t1; ++tt, ++p.it) {
+        const int a = p.it & 1;
+        const uint32_t aph = (p.it >> 1) & 1;
+        const int n0 = tt * BN;
+        const int colh = n0 + half * (BN / 2);
+        // edge tile: positives of this CTA's rows, columns beyond N or rows beyond M (all masked to g = 0)
+        const bool edge = row_edge || ((d_lo + BM - 1 >= n0) && (d_lo < (long long)n0 + BN)) || (n0 + BN > ncols);
+        ptx::mbar_wait(c.bar_tfull + 8 * a, aph);
+        ptx::tc_fence_after();
+        const uint32_t taddr = c.tmem_base + a * BN + half * (BN / 2) + (uint32_t(q * 32) << 16);
+        uint32_t stg = 0;
+        auto piece = [&](const uint32_t (&r)[16], int pi) {
+            const int col0 = colh + pi * 16;
+            if ((pi & 1) == 0) {
+                // half buffers of 32 columns, two pieces each: at most one older bulk store may still read this warp's
+                // other half
+                if (lane == 0) ptx::tma_store_wait_read<1>();
+                __syncwarp();
+                stg = stg0 + (p.stg_use & 1) * (STG_BYTES / 2);
+            }
+            float g[16];
+            if (edge) sig_grad16<true>(r, sc2, t2, p2e, col0, ncols, dcol, row_ok, sg, sgx, g);
+            else sig_grad16<false>(r, sc2, t2, p2e, col0, ncols, dcol, row_ok, sg, sgx, g);
+            grad16_store<false, true>(g, stg, 0, lane, (pi & 1) * 2);
+            if (pi & 1) {
+                ptx::fence_proxy_async_smem();
+                __syncwarp();
+                if (lane == 0) {
+                    ptx::tma_store_2d(tmC, stg, col0 - 16, c_row_off);
+                    ptx::tma_store_commit();
+                }
+                ++p.stg_use;
+            }
+        };
+        uint32_t ra[16], rb[16];
+        ptx::tmem_ld_32x16(taddr, ra);
+        ptx::tmem_ld_wait();
+#pragma unroll
+        for (int pi = 0; pi < 8; pi += 2) {
+            ptx::tmem_ld_32x16(taddr + (pi + 1) * 16, rb);
+            piece(ra, pi);
+            ptx::tmem_ld_wait();
+            if (pi + 2 < 8) {
+                ptx::tmem_ld_32x16(taddr + (pi + 2) * 16, ra);
+            } else {
+                ptx::tc_fence_before();
+                __syncwarp();
+                if (lane == 0) ptx::mbar_arrive_leader(c.bar_tempty + 8 * a);
+            }
+            piece(rb, pi + 1);
+            if (pi + 2 < 8) ptx::tmem_ld_wait();
+        }
+    }
+    if (row_ok) {
+        const size_t slot = (size_t)(part * PARTS_PER_UNIT + half) * args.M + row;
+        args.part_a[slot] = sg;
+        args.part_b[slot] = sgx;
+    }
+}
+
+// Recompute of one G panel: rows of X resident (ARES, K <= 512) or streamed with Y (K > 512), G tiles out through TMA.
+template <bool ARES>
+__global__ void __launch_bounds__(NUM_THREADS, 1)
+siglip_grad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
+                   const __grid_constant__ CUtensorMap tmC, const SigArgs args, const SweepGeom geom) {
+    constexpr int STAGES = sig_grad_stages(ARES);
+    const Cta c = cta_setup<STAGES, GRAD_SWEEP_STG, (ARES ? ARES_KB : STAGES) * A_STAGE_BYTES>();
+    const int cluster = blockIdx.x >> 1, n_clusters = gridDim.x >> 1;
+    Pipe p;
+    if (c.warp == 0) {
+        if (c.lane == 0) {
+            ptx::prefetch_tmap(&tmA);
+            ptx::prefetch_tmap(&tmB);
+            sweep_produce<STAGES, ARES>(c, p, &tmA, &tmB, geom, cluster, n_clusters);
+        }
+    } else if (c.warp == 1) {
+        if (c.lane == 0 && c.leader) sweep_mma<STAGES, 0, ARES>(c, p, geom, cluster, n_clusters);
+    } else {
+        const long long total = (long long)geom.m_pairs * geom.n_tiles;
+        SweepWalk w(geom, cluster, n_clusters);
+        SweepUnit un;
+        while (w.next(un)) {
+            const int part = cluster - sweep_cluster_of(total, (long long)un.m_pair * geom.n_tiles, n_clusters);
+            sig_grad_epilogue_unit(c, p, &tmC, args, 2 * un.m_pair + int(c.cta_rank), part, un.t0, un.t1);
+        }
+        epilogue_drain(c);
+    }
+    cta_teardown(c);
+}
+
 }  // namespace clipk
