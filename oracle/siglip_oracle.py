@@ -45,3 +45,23 @@ def siglip_world(images, texts, logit_scale, logit_bias=0.0, grad_output=1.0):
 
 def siglip_single(image, text, logit_scale, logit_bias=0.0, grad_output=1.0):
     return siglip_world([image], [text], logit_scale, logit_bias, grad_output)[0]
+
+
+def siglip_block(image, text_all, logit_scale, logit_bias=0.0, grad_output=1.0, diag_offset=0):
+    """One rank's block as clipk_siglip_forward / _backward see it: image [b, d], text_all [N, d] (every rank's text
+    rows), the positive of row i at column diag_offset + i.  Returns SigLipGrads whose d_text is the block's UNREDUCED
+    [N, d] partial go (s/b) G^T X; summing the blocks of all ranks and taking rows [r*b, (r+1)*b) gives siglip_world's
+    d_text of rank r."""
+    X, Y = np.asarray(image, dtype=np.float64), np.asarray(text_all, dtype=np.float64)
+    b, N = X.shape[0], Y.shape[0]
+    s, t, go = float(logit_scale), float(logit_bias), float(grad_output)
+    i, j = np.arange(b), np.arange(b) + int(diag_offset)
+    assert 0 <= diag_offset and diag_offset + b <= N
+    dots = X @ Y.T
+    L = s * dots + t
+    z = -np.ones_like(L)
+    z[i, j] = 1.0
+    G = expit(L)
+    G[i, j] = -expit(-L[i, j])
+    return SigLipGrads(np.logaddexp(0.0, -z * L).sum() / b, go * s / b * (G @ Y), go * s / b * (G.T @ X),
+                       go / b * (G * dots).sum(), go / b * G.sum())

@@ -97,6 +97,82 @@ def test_oracle_matches_open_clip_transcription(world):
         assert np.abs(d_text[r].numpy() - ref[r].d_text).max() <= 1e-12 * np.abs(ref[r].d_text).max()
 
 
+@pytest.mark.parametrize("world", [1, 3])
+def test_oracle_blocks_sum_to_world(world):
+    """siglip_block on rank r's geometry (X = images[r], all text rows, positives at r*b + i): the loss, d_image,
+    d_scale and d_bias of siglip_world's rank r, and the [N, d] text partials summed over the ranks its d_text."""
+    b, d, s, t, go = 5, 12, 9.0, -4.0, -1.3
+    feats = [_features(b, d, 200 + r, scale=1.2) for r in range(world)]
+    images, texts = [f[0].numpy() for f in feats], [f[1].numpy() for f in feats]
+    ref = SO.siglip_world(images, texts, s, t, go)
+    text_all = np.concatenate(texts)
+    blocks = [SO.siglip_block(images[r], text_all, s, t, go, diag_offset=r * b) for r in range(world)]
+    d_text = sum(blk.d_text for blk in blocks)
+    assert d_text.shape == (world * b, d)
+    for r, (blk, g) in enumerate(zip(blocks, ref)):
+        assert abs(blk.loss - g.loss) <= 1e-13 * abs(g.loss)
+        for got, want in ((blk.d_image, g.d_image), (d_text[r * b:(r + 1) * b], g.d_text)):
+            assert np.abs(got - want).max() <= 1e-13 * np.abs(want).max()
+        assert abs(blk.d_scale - g.d_scale) <= 1e-13 * max(abs(g.d_scale), 1.0)
+        assert abs(blk.d_bias - g.d_bias) <= 1e-13 * max(abs(g.d_bias), 1.0)
+
+
+def _sig_struct(rows=300, cols=600, d=128, diag_offset=300):
+    """A clipk_siglip that passes every argument check: non-null fake device pointers, 16-byte aligned rows, a 256-byte
+    aligned workspace of exactly clipk_siglip_workspace_bytes().  Only ever handed to the library without a GPU, where
+    the first CUDA call fails before anything is dereferenced."""
+    import ctypes
+    from clipk import _lib
+    c = _lib.Siglip()
+    c.rows, c.cols, c.d = rows, cols, d
+    c.x, c.ldx, c.y, c.ldy = 0x100000, d, 0x200000, d
+    c.logit_scale, c.logit_bias, c.state, c.diag_offset = 0x300000, 0x300100, 0x300200, diag_offset
+    c.workspace = 0x1000000
+    c.workspace_bytes = _lib.load().clipk_siglip_workspace_bytes(ctypes.byref(c))
+    return c
+
+
+def test_siglip_abi_validates_arguments_without_a_gpu():
+    """clipk_siglip_forward / _backward check their arguments before any CUDA call: each bad field gives its own return
+    code, and a struct that passes every check gets as far as the device query (which fails without a GPU)."""
+    import ctypes
+    from clipk import _lib
+    lib = _lib.load()
+    if torch.cuda.is_available():
+        pytest.skip("GPU present")
+    EINVAL, EUNSUPPORTED, EWORKSPACE = -1, -2, -4
+
+    def rc(**fields):
+        c = _sig_struct()
+        for k, v in fields.items():
+            setattr(c, k, v)
+        return lib.clipk_siglip_forward(ctypes.byref(c)), lib.clipk_siglip_backward(ctypes.byref(c))
+
+    ok = _sig_struct()
+    assert ok.workspace_bytes > 0
+    assert lib.clipk_siglip_forward(ctypes.byref(ok)) not in (0, EINVAL, EUNSUPPORTED, EWORKSPACE)
+    ok.grad_out = 0x300300
+    ok.d_bias = 0x300400
+    assert lib.clipk_siglip_backward(ctypes.byref(ok)) not in (0, EINVAL, EUNSUPPORTED, EWORKSPACE)
+    ok.grad_out = None
+    assert lib.clipk_siglip_backward(ctypes.byref(ok)) == EINVAL                 # grad_out is required
+    assert rc(d=100) == (EUNSUPPORTED, EUNSUPPORTED)
+    assert rc(diag_offset=301) == (EINVAL, EINVAL)                               # diag_offset + rows > cols
+    assert rc(diag_offset=-1) == (EINVAL, EINVAL)
+    assert rc(cols=299, diag_offset=0) == (EINVAL, EINVAL)
+    assert rc(ldx=64) == (EINVAL, EINVAL)                                        # ldx < d
+    assert rc(ldy=127) == (EINVAL, EINVAL)
+    assert rc(x=0x100008) == (EINVAL, EINVAL)                                    # x off 16-byte alignment
+    assert rc(workspace=0x1000080) == (EINVAL, EINVAL)                           # workspace off 256-byte alignment
+    assert rc(workspace_bytes=ok.workspace_bytes - 1) == (EWORKSPACE, EWORKSPACE)
+    assert rc(state=None) == (EINVAL, EINVAL)
+    assert rc(rows=0) == (EINVAL, EINVAL)
+    c = _sig_struct()
+    c.rows = 0
+    assert lib.clipk_siglip_workspace_bytes(ctypes.byref(c)) == 0
+    assert lib.clipk_siglip_workspace_bytes(None) == 0
+
+
 def _case(name, rank, world):
     """(features, s, t, grad_output, dtype) of a named case on `rank`"""
     d = 72 if name == "odd_width" else 64
